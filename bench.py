@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- fused indicator suite throughput (symbol.bars/s) on B200, one JSON line.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c2|c3|c5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c2|c3|c5] [--dump-outputs DIR]
 
 A "step" is one pass of the fused 15-indicator / 21-output suite over one synthetic random-walk
 OHLCV panel already resident in HBM.  N > 1 is launched by torchrun, one process per GPU; symbols
@@ -44,6 +44,8 @@ N_IN, N_OUT = 4, 21
 ALGO_BYTES_PER_SYMBOL_BAR = 8 * (N_IN + N_OUT)          # 200 B (SURVEY.md 8d); validity bits (+2.6 B) not counted
 METRIC = "symbol_bars_per_sec_fused_indicator_suite"
 UNIT = "symbol*bars/s"
+DUMP_BYTES = 64_000_000                                  # --dump-outputs: all files together stay below this
+DUMP_SEED = 0x5EED
 
 
 def measured_peak():
@@ -154,6 +156,38 @@ def synth_host_sample(n_symbols, n_bars, seed=0xC0FFEE):
     import synth
     d = synth.ohlcv(n_symbols, n_bars, seed=seed)
     return d["close"], d["high"], d["low"], d["volume"]
+
+
+def dump_outputs(panel, out_dir):
+    """Writes the 21 result columns of the panel's last suite run as a caller receives them, values and validity:
+    out_dir/<output>.npy, float64 [symbols, bars], 0.0 where the value is null, and out_dir/<output>_valid.npy, float32,
+    1.0 where the validity bit is set and 0.0 where it is clear.  Covers a fixed seeded sample of the panel's symbols
+    small enough to keep the files within DUMP_BYTES.  Read from the tiled device planes."""
+    import devread
+    from polars_quant_b200 import _native as NV
+    S, N = panel.n_symbols, panel.n_bars
+    k = min(S, (DUMP_BYTES - 2 * 4096 * N_OUT) // (N_OUT * N * (8 + 4)))
+    if k < 1:
+        raise SystemExit("--dump-outputs: one symbol's %d outputs over %d bars exceed %d bytes" % (N_OUT, N, DUMP_BYTES))
+    syms = np.sort(np.random.default_rng(DUMP_SEED).choice(S, size=k, replace=False))
+    _, bars_padded = panel.tiled_shape()
+    os.makedirs(out_dir, exist_ok=True)
+    for j, name in enumerate(NV.OUTPUT_NAMES[:N_OUT]):
+        vals_ptr = NV.lib().pqb_panel_device_output(panel._h, j)
+        bits_ptr = NV.lib().pqb_panel_device_validity(panel._h, j)
+        out = np.empty((k, N), dtype=np.float64)
+        valid = np.empty((k, N), dtype=bool)
+        for b in np.unique(syms // 32):
+            rows = np.flatnonzero(syms // 32 == b)
+            vals = devread.read_block(vals_ptr, int(b), bars_padded, N)
+            ok = devread.read_validity_rows(bits_ptr, int(b) * 32, min(32, S - int(b) * 32), panel.validity_pitch, N)
+            lanes = syms[rows] % 32
+            valid[rows] = ok[lanes]
+            out[rows] = np.where(ok[lanes], vals[lanes], 0.0)
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+        np.save(os.path.join(out_dir, name + "_valid.npy"), valid.astype(np.float32))
+    sys.stderr.write("[bench] wrote %d outputs of symbols %s (of %d) x %d bars to %s\n"
+                     % (N_OUT, syms.tolist(), S, N, out_dir))
 
 
 def run_reference(args, shape, rank, world):
@@ -288,7 +322,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the fused suite's 21 outputs of the last step for a fixed seeded sample of "
+                         "symbols as DIR/<output>.npy (float64, 0.0 where null) and DIR/<output>_valid.npy (float32, 1.0 where "
+                         "valid), under 64 MB in all; rank 0's share under torchrun")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs writes the fused suite's outputs: --impl ours with --workload %s" % " or ".join(sorted(WORKLOADS)))
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -374,6 +414,8 @@ def main():
     fused_ms_avg = ms_fused / args.steps
     # roofline of THIS rank's launch (the slowest rank's duration): algorithmic bytes of its own share
     achieved = ALGO_BYTES_PER_SYMBOL_BAR * S * N / (fused_ms_avg * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(panel, args.dump_outputs)
     panel.close()
 
     # ---- end to end through the public column API ------------------------------------------------------------------

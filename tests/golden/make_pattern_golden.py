@@ -6,13 +6,13 @@ The reference cannot be compiled in this image (no cargo/rustc), but src/talib/p
 a tiny, regular subset of Rust: per function one `for i in K..n { let x = <expr>; ... if m { out[i] = V; } }`
 loop over plain f64 comparisons, plus a dozen one-line helper predicates.  This script translates that
 text to Python MECHANICALLY, token for token (`&&` -> `and`, `||` -> `or`, `let` dropped, braces ->
-indentation, `(a).abs()` -> `abs(a)`, `a.min(b)` -> `min(a, b)`), at generation time, from
-/root/reference, and runs it on the candle panel below -- so the vectors are the reference's own
+indentation, `(a).abs()` -> `abs(a)`, `a.min(b)` -> `min(a, b)`), at generation time, from a checkout
+of the original, and runs it on the candle panel below -- so the vectors are the reference's own
 arithmetic (Python floats are IEEE f64, comparisons identical), not a hand restatement.  Nothing of the
 translated source is stored: only this script, the seeds and the outputs travel.  Python's
 `min`/`max` differ from Rust's f64::min/max only for NaN operands; the panel has none.
 
-usage (in the build container, where /root/reference exists):
+usage (POLARS_QUANT_REFERENCE set to a checkout of the original polars-quant):
     python tests/golden/make_pattern_golden.py            # writes tests/golden/candle_golden.npz
 """
 from __future__ import annotations
@@ -23,7 +23,9 @@ from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference/src/talib")
+from rustexec import reference_root
+
+REF = reference_root() / "src" / "talib"
 OUT = Path(__file__).resolve().parent / "candle_golden.npz"
 
 

@@ -6,8 +6,8 @@ maturin / polars; the snapshot does not even type-check -- SURVEY.md facts 2-3).
 however, plain scalar loops in a small subset of Rust, so this script runs them with the interpreter in
 tests/golden/rustexec/ (parser + evaluator + a model of the few polars / std containers they touch):
 
-    /root/reference/src/talib/{overlap,momentum,volatility,volume,price}.rs      -- read at generation time
-    /root/reference/python/polars_quant/talib/*.py                               -- imported verbatim
+    src/talib/{overlap,momentum,volatility,volume,price}.rs      -- read at generation time
+    python/polars_quant/talib/*.py                               -- imported verbatim
 
 Every vector below is therefore the reference's own arithmetic in the reference's own operation order (IEEE
 f64, true fma for mul_add, release-profile usize wrap-around), including its panics (`err` = 2: the process
@@ -15,7 +15,7 @@ would abort) and its PolarsResult errors (`err` = 1).  The only definitions that
 the frozen decisions D1 (calc_rma, undefined in the snapshot) and D2 (slice-style calc_ema / calc_sma), see
 rustexec/ref_exec.py; the functions that go through D1 are listed in `d1_functions` inside the file.
 
-Run in the build container (where /root/reference exists):
+Run with POLARS_QUANT_REFERENCE set to a checkout of the original polars-quant (the paths above are relative to it):
     python tests/golden/make_ref_golden.py            # writes tests/golden/talib_ref_golden.npz
     python tests/golden/make_ref_golden.py --check    # re-executes and compares with the committed file
 """

@@ -22,13 +22,11 @@ from __future__ import annotations
 import importlib
 import sys
 import types
-from pathlib import Path
 
 from . import polars_model as M
+from . import reference_root
 from .polars_model import Some
 from .ref_exec import Reference, column, literal
-
-REF_PY = Path("/root/reference/python/polars_quant")
 
 
 class Expr:
@@ -108,10 +106,11 @@ class Shims:
         saved = {k: sys.modules.get(k) for k in ("polars", "polars.plugins")}
         sys.modules["polars"], sys.modules["polars.plugins"] = pl, plugins
         try:
+            ref_py = reference_root() / "python" / "polars_quant"
             pkg = types.ModuleType("_refpq")
-            pkg.__path__ = [str(REF_PY)]
+            pkg.__path__ = [str(ref_py)]
             talib = types.ModuleType("_refpq.talib")
-            talib.__path__ = [str(REF_PY / "talib")]
+            talib.__path__ = [str(ref_py / "talib")]
             sys.modules["_refpq"], sys.modules["_refpq.talib"] = pkg, talib
             for m in ("overlap", "momentum", "volatility", "volume", "price"):
                 setattr(talib, m, importlib.import_module(f"_refpq.talib.{m}"))

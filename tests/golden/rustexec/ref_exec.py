@@ -1,6 +1,6 @@
 """Runs the reference's plugin functions from their own source text.  TEST INFRASTRUCTURE.
 
-`Reference()` parses /root/reference/src/talib/{overlap,momentum,volatility,volume,price,pattern}.rs and
+`Reference()` parses src/talib/{overlap,momentum,volatility,volume,price,pattern}.rs of the original and
 exposes `call(fn_name, columns, params=..., kwargs=...)`, which builds the `inputs: &[Series]` (+ the serde
 kwargs struct) exactly as polars would hand them to `#[polars_expr] fn <fn_name>` and returns the result
 columns as (values, validity) numpy pairs -- or raises `ReferenceError` (a `PolarsResult::Err`) /
@@ -21,11 +21,11 @@ from pathlib import Path
 import numpy as np
 
 from . import polars_model as M
+from . import reference_root
 from .polars_model import Err, Ok, RustPanic, Some
 from .rs_eval import Interp, RustRuntimeError
 from .rs_parse import parse_rust
 
-REF_SRC = Path("/root/reference/src/talib")
 MODULES = ("overlap", "momentum", "volatility", "volume", "price", "pattern")
 
 
@@ -95,7 +95,8 @@ def column(ca):
 
 
 class Reference:
-    def __init__(self, src: Path = REF_SRC, modules=MODULES):
+    def __init__(self, src: Path | None = None, modules=MODULES):
+        src = src or reference_root() / "src" / "talib"
         self.interp = Interp()
         self.interp.extern["calc_rma"] = calc_rma
         self.where = {}

@@ -5,7 +5,7 @@ TEST INFRASTRUCTURE (golden-vector generation only).  The reference cannot be co
 under tests/golden/ are made by EXECUTING the reference's own source text with the small interpreter
 in this directory: this file turns the text into a syntax tree, rs_eval.py walks it, polars_model.py
 models the handful of polars / std containers the text touches.  Nothing of the reference's text is
-stored in the repo; it is read from /root/reference at generation time.
+stored in the repo; it is read from a checkout of the original at generation time (rustexec.reference_root).
 
 Supported: `use` (skipped), attributes (skipped), `struct` with named fields, `fn` (also nested),
 `let` with patterns / type annotations, `if` / `if let` / `else`, `match` with guards, `while` /

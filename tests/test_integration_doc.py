@@ -44,7 +44,7 @@ def test_generated_binding_covers_every_declared_function_and_struct_field():
     assert "outputs_mask: u64" in block and "pub donchian_period: i32" in block
 
 
-def test_ctypes_mirror_matches_the_header_layouts():
+def test_ctypes_mirror_matches_the_header_layouts(tmp_path):
     from polars_quant_b200 import _native as N
     for struct, mirror in (("pqb_suite_params", N.SuiteParams), ("pqb_col_ref", N.ColRef), ("pqb_col", N.Col),
                            ("pqb_out_col", N.OutCol), ("pqb_candle_params", N.CandleParams)):
@@ -58,8 +58,7 @@ def test_ctypes_mirror_matches_the_header_layouts():
                 assert ct is CTYPES[ctype.replace("const ", "")], (struct, name, ctype)
     # and the sizes the C compiler gives the same structs
     src = '#include "%s"\n#include <stdio.h>\nint main(void){printf("%%zu %%zu %%zu %%zu %%zu", sizeof(pqb_suite_params), sizeof(pqb_col_ref), sizeof(pqb_col), sizeof(pqb_out_col), sizeof(pqb_candle_params));return 0;}' % G.HEADER
-    exe = ROOT / "tests" / "_sizes.out"
+    exe = tmp_path / "sizes.out"
     subprocess.run(["gcc", "-x", "c", "-", "-o", str(exe)], input=src.encode(), check=True)
     sizes = [int(x) for x in subprocess.run([str(exe)], capture_output=True, check=True).stdout.split()]
-    exe.unlink()
     assert sizes == [C.sizeof(N.SuiteParams), C.sizeof(N.ColRef), C.sizeof(N.Col), C.sizeof(N.OutCol), C.sizeof(N.CandleParams)]

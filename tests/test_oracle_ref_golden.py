@@ -84,9 +84,11 @@ def test_first_valid_index_contract_of_the_reference():
     assert first("A/STOCHF_5_3/0/ok") == 4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/talib"), reason="the reference tree exists only in the build container")
+@pytest.mark.skipif(not os.environ.get("POLARS_QUANT_REFERENCE") or
+                    not os.path.isdir(os.path.join(os.environ["POLARS_QUANT_REFERENCE"], "src", "talib")),
+                    reason="needs POLARS_QUANT_REFERENCE: a checkout of the original polars-quant")
 def test_golden_file_is_what_the_reference_text_produces_today():
-    """Re-executes a sample of the calls from /root/reference and compares with the committed file (provenance)."""
+    """Re-executes a sample of the calls from the original's source text and compares with the committed file (provenance)."""
     import sys
     sys.path.insert(0, str(refgolden.ROOT / "tests" / "golden"))
     from rustexec.ref_exec import Reference, series

@@ -1,8 +1,9 @@
 """The reference-facing name layer (polars_quant_b200/talib.py) against the reference's own Python shims
 (python/polars_quant/talib/*.py): every shim name of the hot path and its "next" rows exists here with the same parameter
-names and defaults.  Reads the reference's files where they exist (the build container); on a box without them only the
-committed expectations are checked."""
+names and defaults.  Reads the reference's files from a checkout of the original named by POLARS_QUANT_REFERENCE; without
+one only the committed expectations are checked."""
 import inspect
+import os
 import re
 from pathlib import Path
 
@@ -10,7 +11,7 @@ import pytest
 
 from polars_quant_b200 import talib
 
-REF = Path("/root/reference/python/polars_quant/talib")
+REF = Path(os.environ.get("POLARS_QUANT_REFERENCE", ""), "python", "polars_quant", "talib")
 # names the reference defines that are out of scope here (SURVEY.md section 2 / DESIGN.md section 8)
 OUT_OF_SCOPE = {"HT_DCPERIOD", "HT_DCPHASE", "HT_PHASOR", "HT_SINE", "HT_TRENDLINE", "HT_TRENDMODE", "MAMA", "MAVP", "SAR", "SAREXT"}
 NOT_BUILT = {"WMA", "DEMA", "T3", "KAMA", "APO", "PPO", "AROONOSC"}
@@ -29,7 +30,8 @@ def test_every_pattern_and_price_name_is_defined():
             getattr(talib, n)(None)
 
 
-@pytest.mark.skipif(not REF.exists(), reason="the reference tree is only present in the build container")
+@pytest.mark.skipif(not os.environ.get("POLARS_QUANT_REFERENCE") or not REF.is_dir(),
+                    reason="needs POLARS_QUANT_REFERENCE: a checkout of the original polars-quant")
 def test_names_parameters_and_defaults_match_the_reference_shims():
     checked = 0
     for f in sorted(REF.glob("*.py")):

@@ -245,6 +245,20 @@ def lib() -> C.CDLL:
                               C.c_double, C.c_void_p]
         L.pqb_price.argtypes = [C.c_void_p, C.c_int, C.POINTER(Col), C.POINTER(Col), C.POINTER(Col), C.POINTER(Col),
                                 C.POINTER(OutCol)]
+        # live panels
+        L.pqb_live_create.argtypes = [C.c_void_p, C.POINTER(SuiteParams), C.c_uint64, C.c_int64, C.POINTER(C.c_void_p)]
+        L.pqb_live_destroy.argtypes = [C.c_void_p]
+        L.pqb_live_destroy.restype = None
+        L.pqb_live_bars.argtypes = [C.c_void_p]
+        L.pqb_live_bars.restype = C.c_int64
+        L.pqb_live_state_bytes.argtypes = [C.c_void_p]
+        L.pqb_live_state_bytes.restype = C.c_int64
+        L.pqb_live_push.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 8 + [C.c_int]
+        L.pqb_live_host_output.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_live_host_output.restype = C.c_void_p
+        L.pqb_live_host_validity.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_live_host_validity.restype = C.c_void_p
+        L.pqb_live_last_push_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         _lib = L
     return _lib
 

@@ -2567,3 +2567,4 @@ extern "C" int pqb_multi_run_host(pqb_multi *m, const pqb_suite_params *params) 
 #include "shims_host.inc"
 #include "signals_host.inc"
 #include "info_host.inc"
+#include "live_host.inc"

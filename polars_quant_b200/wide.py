@@ -435,6 +435,32 @@ class WidePanel:
         lap("assemble_table_ms")
         return out
 
+    # ---- live: append new rows to the computed table ----
+    def live(self, params: N.SuiteParams | None = None, outputs=None, max_push_bars: int = 64, devices=None) -> "WideLive":
+        """A live panel primed from this table (include/pqb200.h "live panels"): `.push(rows)` takes k new rows in the
+        table's own `date` + `{symbol}_{field}` shape and returns `date` + `{symbol}_{output}` for those rows -- the
+        columns, names and values `suite()` of the concatenated table gives for them.  One GPU (`devices` is refused)."""
+        if devices:
+            raise NotImplementedError("live panels run on one GPU: multi-GPU live panels are not built")
+        symbols, cols = split_columns(self.table, SUITE_FIELDS)
+        symbols = [s for s in symbols if all(s in cols[f] for f in SUITE_FIELDS)]
+        if not symbols:
+            raise ValueError("no symbol has all of " + ", ".join("{symbol}_" + f for f in SUITE_FIELDS))
+        params = params or N.default_params()
+        names = list(outputs) if outputs is not None else N.OUTPUT_NAMES[:N.N_SUITE_OUTPUTS]
+        omask = sum(1 << N.OUTPUT_NAMES.index(n) for n in names)
+        sym, fld = self._suite_map(symbols, cols)
+        p = Panel(len(symbols), self.n_bars, engine=self.engine or get_engine(0), outputs_mask=0, host_staging=2)
+        try:
+            arr, sch = self._record_batch_cached()
+            N.check(N.lib().pqb_panel_set_record_batch(p._h, C.byref(arr), C.byref(sch), sym.ctypes.data, fld.ctypes.data, 0))
+            p.upload()
+            from .live import LivePanel
+            lp = LivePanel(p, params, omask, max_push_bars)
+        finally:
+            p.close()
+        return WideLive(lp, symbols, {f: cols[f] for f in SUITE_FIELDS}, sorted(names, key=N.OUTPUT_NAMES.index))
+
     # ---- Selector.info(): last-row reductions (README.md:832-851) ----
     def info(self) -> pa.Table:
         """One row per symbol with the README's 15 `Selector.info()` columns: symbol, price, open, high, low, volume,
@@ -509,3 +535,38 @@ class WidePanel:
                                                       [pa.foreign_buffer(bits, vbytes, base), pa.foreign_buffer(vals, self.n_bars * 8, base)]))
                 out_names.append("%s_%s" % (sym, n))
         return pa.table(out_cols, names=out_names)
+
+
+class WideLive:
+    """`WidePanel.live()`: pushes k new rows of the wide table, returns their `date` + `{symbol}_{output}` rows."""
+
+    def __init__(self, live, symbols, cols, outputs):
+        self.live, self.symbols, self._cols, self.outputs = live, symbols, cols, outputs
+
+    @property
+    def bars(self) -> int:
+        return self.live.bars
+
+    def push(self, rows: pa.Table, commit: bool = True) -> pa.Table:
+        k = rows.num_rows
+        vals, valid = {}, {}
+        index = {name: i for i, name in enumerate(rows.column_names)}
+        for f in SUITE_FIELDS:
+            v = np.empty((k, len(self.symbols)), dtype=np.float64)
+            ok = np.empty((k, len(self.symbols)), dtype=bool)
+            for j, s in enumerate(self.symbols):
+                a = _f64(rows.column(index[self._cols[f][s]]))
+                ok[:, j] = ~np.asarray(a.is_null(), dtype=bool) if a.null_count else True
+                v[:, j] = a.to_numpy(zero_copy_only=False)
+            vals[f], valid[f] = v, ok
+        res = self.live.push(vals["close"], vals["high"], vals["low"], vals["volume"], valid=valid, commit=commit)
+        out_cols, out_names = [], []
+        for j, s in enumerate(self.symbols):
+            for o in self.outputs:
+                v, ok = res[o]
+                out_cols.append(pa.array(v[j], type=pa.float64(), mask=~ok[j]))
+                out_names.append("%s_%s" % (s, o))
+        out = pa.table(out_cols, names=out_names)
+        if "date" in index:
+            out = out.add_column(0, "date", rows.column(index["date"]))
+        return out

@@ -28,6 +28,7 @@ IND_EXTRA = {"midpoint": 1 << 15, "adosc": 1 << 16, "mom": 1 << 17, "roc": 1 << 
              "donchian": 1 << 26}
 IND_ALL = (1 << 15) - 1
 IND_FASTK = 1 << 27          # with IND["kdj"]: also store the raw %K line (output "fastk"); opt-in, the general kernel only
+LIVE_NULLS = 1               # pqb_live_create_ex flag: null-aware live panel (include/pqb200.h)
 
 ERR_NAMES = {-1: "PQB_ERR_NO_DEVICE", -2: "PQB_ERR_CUDA", -3: "PQB_ERR_INVALID", -4: "PQB_ERR_UNSUPPORTED",
              -5: "PQB_ERR_NULLS", -6: "PQB_ERR_ALLOC"}
@@ -259,6 +260,10 @@ def lib() -> C.CDLL:
         L.pqb_live_host_validity.argtypes = [C.c_void_p, C.c_int]
         L.pqb_live_host_validity.restype = C.c_void_p
         L.pqb_live_last_push_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
+        L.pqb_live_create_ex.argtypes = [C.c_void_p, C.POINTER(SuiteParams), C.c_uint64, C.c_int64, C.c_uint32,
+                                         C.POINTER(C.c_void_p)]
+        L.pqb_live_host_voided.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_live_host_voided.restype = C.c_void_p
         _lib = L
     return _lib
 

@@ -8,6 +8,11 @@ recompute over the concatenated history.
 
 `full[name][0][:, T:T + k]` of a recompute over T + k bars equals `rows[name][0]`.  push(..., commit=False) previews the
 current, unfinished bar: the rows come back, the state and `bars` stay as they were.
+
+LivePanel(panel, nulls=True) accepts histories with halts, delistings and fields listed on different rows, and pushes
+with any validity pattern.  A null after a field's first valid bar turns the symbol's whole column of macd / rsi / willr /
+midprice (...) null in the reference, history included; after each push `voided` names the columns it did that to:
+{output name: symbol indices}.
 """
 from __future__ import annotations
 
@@ -20,17 +25,25 @@ from . import _native as N
 
 class LivePanel:
     FIELDS = ("close", "high", "low", "volume")
+    nulls = False
+    voided: dict = {}                               # (the last push's; a new dict per push)
 
-    def __init__(self, panel, params: N.SuiteParams | None = None, outputs: int | None = None, max_push_bars: int = 64):
+    def __init__(self, panel, params: N.SuiteParams | None = None, outputs: int | None = None, max_push_bars: int = 64,
+                 nulls: bool = False):
         """`panel`: a Panel whose inputs are on the device (compute / upload / run_host / fill_synthetic).  `outputs`: a
-        mask of output ids (None: the outputs of params.indicators).  The live panel keeps no reference to `panel`."""
+        mask of output ids (None: the outputs of params.indicators).  `nulls`: the null-aware live panel (any validity
+        pattern in the history and the pushes; see `voided`).  The live panel keeps no reference to `panel`."""
+        if not isinstance(nulls, (bool, np.bool_)):
+            raise TypeError("nulls must be True or False, not %r" % (nulls,))
         self.params = params or N.default_params()
         self.n_symbols = panel.n_symbols
         self.max_push_bars = int(max_push_bars)
+        self.nulls = bool(nulls)
+        self.voided = {}
         self.engine = panel.engine                  # (the native engine must outlive the live panel)
         self._h = C.c_void_p()
-        N.check(N.lib().pqb_live_create(panel._h, C.byref(self.params), C.c_uint64(outputs or 0), C.c_int64(max_push_bars),
-                                        C.byref(self._h)))
+        N.check(N.lib().pqb_live_create_ex(panel._h, C.byref(self.params), C.c_uint64(outputs or 0), C.c_int64(max_push_bars),
+                                           C.c_uint32(N.LIVE_NULLS if self.nulls else 0), C.byref(self._h)))
         self.outputs = [k for k in range(N.N_OUTPUTS) if N.lib().pqb_live_host_output(self._h, k)]
 
     def close(self):
@@ -72,7 +85,8 @@ class LivePanel:
     def push(self, close, high=None, low=None, volume=None, valid=None, commit: bool = True):
         """k new bars: each field float64 [k, n_symbols] (or [n_symbols] for one bar); `valid` None (all valid), one bool
         array for every field, or a dict {field: bool array} of the same shape.  Returns {name: (values, validity)} of
-        shape [n_symbols, k] -- the orientation of Panel.outputs()."""
+        shape [n_symbols, k] -- the orientation of Panel.outputs().  Null-aware panels also set `voided`: {output name:
+        indices of the symbols whose earlier rows of that output this push turned null} (a preview's too)."""
         c = self._rows("close", close, None)
         k = c.shape[0]
         if k > self.max_push_bars:
@@ -101,4 +115,12 @@ class LivePanel:
             b = np.ctypeslib.as_array((C.c_uint8 * (k * vb)).from_address(bp)).reshape(k, vb)
             ok = np.unpackbits(b, axis=1, bitorder="little")[:, :self.n_symbols].astype(bool)
             res[N.OUTPUT_NAMES[kk]] = (v.T.copy(), ok.T.copy())
+        voided = {}
+        if self.nulls:
+            for kk in self.outputs:
+                b = np.ctypeslib.as_array((C.c_uint8 * vb).from_address(N.lib().pqb_live_host_voided(self._h, kk)))
+                syms = np.flatnonzero(np.unpackbits(b, bitorder="little")[:self.n_symbols])
+                if len(syms):
+                    voided[N.OUTPUT_NAMES[kk]] = syms
+        self.voided = voided
         return res

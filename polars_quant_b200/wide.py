@@ -436,10 +436,13 @@ class WidePanel:
         return out
 
     # ---- live: append new rows to the computed table ----
-    def live(self, params: N.SuiteParams | None = None, outputs=None, max_push_bars: int = 64, devices=None) -> "WideLive":
+    def live(self, params: N.SuiteParams | None = None, outputs=None, max_push_bars: int = 64, devices=None,
+             nulls: bool = False) -> "WideLive":
         """A live panel primed from this table (include/pqb200.h "live panels"): `.push(rows)` takes k new rows in the
         table's own `date` + `{symbol}_{field}` shape and returns `date` + `{symbol}_{output}` for those rows -- the
-        columns, names and values `suite()` of the concatenated table gives for them.  One GPU (`devices` is refused)."""
+        columns, names and values `suite()` of the concatenated table gives for them.  One GPU (`devices` is refused).
+        nulls=True: the table and the pushed rows may have halted cells; after each push `WideLive.voided` lists the
+        `{symbol}_{output}` columns whose earlier rows that push turned null."""
         if devices:
             raise NotImplementedError("live panels run on one GPU: multi-GPU live panels are not built")
         symbols, cols = split_columns(self.table, SUITE_FIELDS)
@@ -456,7 +459,7 @@ class WidePanel:
             N.check(N.lib().pqb_panel_set_record_batch(p._h, C.byref(arr), C.byref(sch), sym.ctypes.data, fld.ctypes.data, 0))
             p.upload()
             from .live import LivePanel
-            lp = LivePanel(p, params, omask, max_push_bars)
+            lp = LivePanel(p, params, omask, max_push_bars, nulls=nulls)
         finally:
             p.close()
         return WideLive(lp, symbols, {f: cols[f] for f in SUITE_FIELDS}, sorted(names, key=N.OUTPUT_NAMES.index))
@@ -542,6 +545,7 @@ class WideLive:
 
     def __init__(self, live, symbols, cols, outputs):
         self.live, self.symbols, self._cols, self.outputs = live, symbols, cols, outputs
+        self.voided: list[str] = []             # `{symbol}_{output}` columns whose earlier rows the last push made null
 
     @property
     def bars(self) -> int:
@@ -560,6 +564,7 @@ class WideLive:
                 v[:, j] = a.to_numpy(zero_copy_only=False)
             vals[f], valid[f] = v, ok
         res = self.live.push(vals["close"], vals["high"], vals["low"], vals["volume"], valid=valid, commit=commit)
+        self.voided = ["%s_%s" % (self.symbols[j], o) for o in self.outputs for j in self.live.voided.get(o, ())]
         out_cols, out_names = [], []
         for j, s in enumerate(self.symbols):
             for o in self.outputs:

@@ -18,8 +18,8 @@
 //                             REFERENCE'S OWN operation order (fma(alpha, x - y, y), dif = f - s, hist = dif - signal),
 //                             writing every output once
 // Tile 0 (and the tile that holds a chain's seed bar) is the reference's computation itself; later tiles differ from the
-// serial walk only through the rounding of the carried start state (a few ulp of the state, i.e. relative 1e-15 of the
-// price level), inside the north-star tolerance (rel 1e-10 / abs 1e-12) -- tolerance-exact, not bit-exact, like the
+// serial walk only through the rounding of the carried start state (a few ulp of the state): EMA lines within rel 1e-10 /
+// abs 1e-12, MACD lines within that + 4 ulp of the row's largest |close| -- tolerance-exact, not bit-exact, like the
 // time-split panels of split_host.inc, but with no warm-up recomputation: 72 B of traffic per symbol-bar (close read
 // twice) against 64 B algorithmic, whatever the period.
 // Layout: the tiled planes of suite_kernel.cuh ([symbol block][bar][32 symbols]); lane = symbol, one warp = one

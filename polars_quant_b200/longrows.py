@@ -6,8 +6,9 @@ MACD in ONE pass over close, parallel along time (include/pqb200.h "long rows", 
     res = lp.compute()                          # {"ema_12": (values, validity), ..., "macd": ..., "macd_signal": ..., "macd_hist": ...}
 
 Replaces, per symbol, `with_columns([EMA(c, 12), EMA(c, 26), EMA(c, 200), EMA(c, 5000), *MACD(c, 12, 26, 9)])` of the
-reference (README.md:1360-1365): calc_ema overlap.rs:660-730, macd momentum.rs:250-283.  Tolerance-exact (rel 1e-10 /
-abs 1e-12 against the serial reference; the first time tile is bit-exact), like SplitPanel but with no warm-up."""
+reference (README.md:1360-1365): calc_ema overlap.rs:660-730, macd momentum.rs:250-283.  Tolerance-exact, like SplitPanel
+but with no warm-up: the EMA lines within rel 1e-10 / abs 1e-12 of the serial reference, the MACD lines (which cross zero)
+within that plus 4 ulp of the row's largest |close|; the first time tile is bit-exact."""
 from __future__ import annotations
 
 import ctypes as C

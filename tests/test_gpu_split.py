@@ -52,6 +52,24 @@ def test_config3_ema_macd_split_against_the_serial_oracle(pq):
         p.close()
 
 
+def test_ema_and_macd_at_a_high_price_level(pq):
+    """Price level 1e5, where one ulp of the price (1.5e-11) is larger than abs 1e-12: a chunk's warm-up converges to the
+    serial state's own bits, so the MACD lines, which cross zero, still meet rel 1e-10 / abs 1e-12 (measured on a B200:
+    the MACD lines bit-identical to the serial oracle)."""
+    S, NB, period = 5, 400_000, 12
+    close = synth.ohlcv(S, NB, seed=3, sigma=0.0005)["close"] * 1e3
+    om = sum(1 << pqo.OUTPUT_NAMES.index(o) for o in ("ema", "macd", "macd_signal", "macd_hist"))
+    prm = N.default_params(indicators=N.IND["ema"] | N.IND["macd"], ema_period=period)
+    p = pq.SplitPanel(S, NB, chunks=16, warmup=pq.SplitPanel.required_warmup(prm), fields_mask=1, outputs_mask=om)
+    p.set_fields(close=close)
+    p.run_host(prm)
+    for s in range(S):
+        _close_enough("ema", p.get_output(s, pqo.OUTPUT_NAMES.index("ema")), pqo.ema(close[s], period))
+        for name, ref in zip(("macd", "macd_signal", "macd_hist"), pqo.macd(close[s], 12, 26, 9)):
+            _close_enough(name, p.get_output(s, pqo.OUTPUT_NAMES.index(name)), ref)
+    p.close()
+
+
 def test_split_suite_recurrences_and_window_functions(pq):
     S, NB = 4, 60_000
     d = synth.ohlcv(S, NB, seed=8)

@@ -859,6 +859,7 @@ static inline double ema_alpha(int p) { return 2.0 / ((double)p + 1.0); }   // o
 struct Built {
     SuiteArgs a;
     int lead[PQB_N_OUTPUTS];   // first valid index of each output relative to the symbol start
+    int steady_b;              // a.steady_lead of the benchmark groups alone (their own null-aware launch next to optional groups)
 };
 
 static bool split_launch_enabled() {
@@ -1102,6 +1103,7 @@ static int build_args(const pqb_panel *p, const pqb_suite_params *sp, Built *out
             return fail(PQB_ERR_UNSUPPORTED, "midprice period %d (reference: never-expiring deque) is not built", sp->midprice_period);
         A.gmask |= G_MIDPRICE; A.mid_p = sp->midprice_period; bind(PQB_OUT_MIDPRICE, 0);
     }
+    out->steady_b = steady;
     // ---- optional groups (SURVEY.md 8a, not part of the benchmark suite) ----
     auto bind_dyn = [&](int k) { if (want(k)) { A.out[k] = p->d_out[k]; out->lead[k] = NEVER; } };   // validity from the kernel
     if (ind & PQB_IND_MIDPOINT) {
@@ -1484,16 +1486,14 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         // benchmark groups and optional groups together: two launches -- the benchmark groups through their
         // compile-time-specialised kernels (full suite / partial suite), the optional groups through the general one
         // (it re-reads the input planes; the general kernel is 2.4x slower on the benchmark groups than the full-suite
-        // kernel: 50,000 x 5,040 suite + MOM 23.2 ms in one general launch).  Null-aware mode has one kernel for everything.
+        // kernel: 50,000 x 5,040 suite + MOM 23.2 ms in one general launch).  The flagged blocks of a panel with nulls split the
+        // same way, between two null-aware launches (launch_null below).
         const unsigned gb = full.a.gmask & (unsigned)G_ALL, go = full.a.gmask & ~(unsigned)G_ALL;
         int rc;
         // which blocks of the range need the null-aware kernel
         int64_t n_null = 0;
         if (p->nulls_mode)
             for (int64_t b = b0; b < b0 + nb; ++b) n_null += p->h_blk_null[(size_t)b];
-        if (n_null && go)
-            return fail(PQB_ERR_UNSUPPORTED, "midpoint / adosc / mom / roc / cmo / mfi / cci / ... are not built for panels with "
-                                             "interior nulls yet (momentum.rs functions fail on such input in the reference)");
         const int *plain_list = nullptr, *null_list = nullptr;
         // The benchmark suite's null-aware kernel (<FULLS, NULLS> with fast stages) walks a block with a few halted symbols about as fast
         // as the plain kernel does, so flagged blocks simply run through it, beside the plain launch: no gather, no write-back, no
@@ -1607,14 +1607,31 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         // per-block dispatch with both kinds of blocks: the null-aware launch (the longer walk) goes first, on the second stream,
         // and the plain launch runs beside it (8,192 x 5,040 with one halted symbol: 1.6 + 1.9 ms back to back -> side by side)
         static const bool side_by_side = !getenv("PQB_NULLS_CONCURRENT") || atoi(getenv("PQB_NULLS_CONCURRENT")) != 0;
-        bool null_done = false;
-        if (!did_compact && n_null && n_null < nb && side_by_side) {
+        // the flagged blocks.  Next to optional groups the benchmark groups keep a null-aware launch of their own -- the
+        // specialised kernel with fast stages when all 21 suite outputs are bound, as without optional groups -- and the optional
+        // groups, whose null rules have no fast stages, walk the same blocks through the general null-aware kernel.
+        auto launch_null = [&]() -> int {
+            if (gb && go && split_launch_enabled()) {
+                SuiteArgs ab = null_variant(p, full.a), ao = ab;
+                ab.gmask = gb;
+                ab.steady_lead = full.steady_b;
+                for (int k = 0; k < PQB_N_OUTPUTS; ++k) if (outputs_of_groups(go) >> k & 1) ab.out[k] = nullptr;
+                ab.nulls_fast = nulls_fast_ok(ab);
+                ao.gmask = go;
+                if ((rc = layout_rings(ab, p)) || (rc = layout_rings(ao, p))) return rc;      // (subsets of a layout that fits)
+                if ((rc = launch_one(ab, null_list, n_null))) return rc;
+                return launch_one(ao, null_list, n_null);
+            }
             SuiteArgs an = null_variant(p, full.a);
             if (!an.smem_bytes && (rc = layout_rings(an, p))) return rc;
+            return launch_one(an, null_list, n_null);
+        };
+        bool null_done = false;
+        if (!did_compact && n_null && n_null < nb && side_by_side) {
             CU(cudaEventRecord(e->ev_fork, e->stream));       // (after the block lists' copies)
             CU(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
             std::swap(e->stream, e->side);                    // (a null-aware launch_one() touches e->stream only)
-            rc = launch_one(an, null_list, n_null);
+            rc = launch_null();
             std::swap(e->stream, e->side);
             if (rc) return rc;
             null_done = true;
@@ -1633,10 +1650,8 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         if (null_done) {                                      // join the second stream
             CU(cudaEventRecord(e->ev_side, e->side));
             CU(cudaStreamWaitEvent(e->stream, e->ev_side, 0));
-        } else if (!did_compact && n_null) {                  // the flagged blocks: one null-aware launch
-            SuiteArgs an = null_variant(p, full.a);
-            if (!an.smem_bytes && (rc = layout_rings(an, p))) return rc;
-            if ((rc = launch_one(an, null_list, n_null))) return rc;
+        } else if (!did_compact && n_null) {
+            if ((rc = launch_null())) return rc;
         }
     }
 #ifdef PQB_DEBUG_SMID
@@ -2135,19 +2150,16 @@ extern "C" int pqb_selftest_divsqrt(pqb_engine *e, const double *a, const double
 // ---------------------------------------------------------------------------------------
 // single-column entry points: one reference plugin call on one column
 // ---------------------------------------------------------------------------------------
-struct ColCheck { int64_t lead; bool any_null; bool interior; };
+struct ColCheck { bool any_null; };
 static ColCheck scan_col(const pqb_col *c) {
-    ColCheck r{0, false, false};
+    ColCheck r{false};
     if (!c->validity) return r;
-    while (r.lead < c->len && !bit_at(c->validity, c->offset + r.lead)) ++r.lead;
-    r.any_null = r.lead > 0;
-    for (int64_t i = r.lead; i < c->len; ++i)
-        if (!bit_at(c->validity, c->offset + i)) { r.any_null = true; r.interior = true; break; }
+    for (int64_t i = 0; i < c->len; ++i)
+        if (!bit_at(c->validity, c->offset + i)) { r.any_null = true; break; }
     return r;
 }
 
-enum NullPolicy { NP_SHIFT, NP_ERR, NP_LEAD };   // overlap/volatility/volume functions skip nulls; momentum.rs errors;
-                                                  // NP_LEAD: a null-skipping function built for leading nulls only
+enum NullPolicy { NP_SHIFT, NP_ERR };   // overlap/volatility/volume functions skip nulls; momentum.rs errors
 
 static int run_single(pqb_engine *e, const pqb_col *const *cols, const int *fields, int n_cols, NullPolicy np,
                       const pqb_suite_params *sp, const int *outs, pqb_out_col *const *dst, int n_out) {
@@ -2165,9 +2177,6 @@ static int run_single(pqb_engine *e, const pqb_col *const *cols, const int *fiel
         ColCheck cc = scan_col(cols[i]);
         if (cc.any_null && np == NP_ERR)
             return fail(PQB_ERR_NULLS, "chunked array is not contiguous (input %d has nulls; reference: cont_slice()?)", i);
-        if (cc.interior && np == NP_LEAD)
-            return fail(PQB_ERR_UNSUPPORTED, "input %d has interior / trailing nulls: the reference skips null bars here, this build "
-                                             "handles leading nulls only for this function", i);
     }
     if (n == 0) return PQB_OK;
     // device required from here on
@@ -2382,14 +2391,14 @@ extern "C" int pqb_midprice(pqb_engine *e, const pqb_col *h, const pqb_col *l, i
 extern "C" int pqb_midpoint(pqb_engine *e, const pqb_col *real, int32_t tp, pqb_out_col *out) {
     pqb_suite_params sp = only(PQB_IND_MIDPOINT); sp.midpoint_period = tp;
     const pqb_col *c[] = {real}; const int f[] = {PQB_CLOSE}; const int o[] = {PQB_OUT_MIDPOINT}; pqb_out_col *d[] = {out};
-    return run_single(e, c, f, 1, NP_LEAD, &sp, o, d, 1);     // (null-skipping in the reference; interior nulls not built yet)
+    return run_single(e, c, f, 1, NP_SHIFT, &sp, o, d, 1);    // (overlap.rs:180-278: a null bar emits null, the window skips it)
 }
 extern "C" int pqb_adosc(pqb_engine *e, const pqb_col *h, const pqb_col *l, const pqb_col *cl, const pqb_col *v,
                          int32_t fp, int32_t slp, pqb_out_col *out) {
     pqb_suite_params sp = only(PQB_IND_ADOSC); sp.adosc_fast = fp; sp.adosc_slow = slp;
     const pqb_col *c[] = {h, l, cl, v}; const int f[] = {PQB_HIGH, PQB_LOW, PQB_CLOSE, PQB_VOLUME};
     const int o[] = {PQB_OUT_ADOSC}; pqb_out_col *d[] = {out};
-    return run_single(e, c, f, 4, NP_LEAD, &sp, o, d, 1);     // (calc_ad / calc_ema skip null bars; interior nulls not built yet)
+    return run_single(e, c, f, 4, NP_SHIFT, &sp, o, d, 1);    // (calc_ad / calc_ema skip null bars)
 }
 extern "C" int pqb_mom(pqb_engine *e, const pqb_col *real, int32_t tp, pqb_out_col *out) {
     pqb_suite_params sp = only(PQB_IND_MOM); sp.mom_period = tp;

@@ -15,6 +15,9 @@
 // two-level form (Ext2 below: 2 sqrt(p)-sized arrays in shared memory, raw rows re-read from the input planes by TMA).
 // No producer warp: the unit warp that is LAST to leave a stage refills it (one shared-memory counter per stage), so every
 // warp of the CTA computes and a CTA of U units costs U warps of registers.
+// Null-aware variant (window_suite_kernel<..., true>, for the symbol blocks of a panel with halts, delistings or fields listed
+// on different rows): each stage also carries the stage's input validity words, every unit walks the step_nulls() body of the
+// suite role it mirrors (Role3 / Role5 / Role6 in suite_kernel.cuh) and every output line leaves one ballot word per bar.
 #pragma once
 #include "suite_kernel.cuh"
 
@@ -56,8 +59,15 @@ struct WinArgs {
     int relaxed_wait;                  // sleep between failed tries of the stage wait
     int block_major;                   // CTA order: the groups of one symbol block next to each other (they share its input rows in L2)
     int steady_lead;                   // a lane is past every warm-up once t - start >= steady_lead
-    int n_symbols, n_bars, n_blocks, bars_padded;
+    int n_symbols, n_bars, n_blocks, bars_padded;   // (n_blocks: the blocks of this launch)
+    const int *blist;                  // block i of the launch is blist[i] (nullptr: block i)
+    // null-aware variant only
+    const uint32_t *vmask;             // input validity words [block][bar][4] (pack_mask_kernel)
+    const uint8_t *symflags;           // per symbol: bit f = field f has a null after its first valid bar
+    uint32_t *ovm[W_MAX_TOTAL][4];     // unit i, line q: ballot words [block][bar]
+    int mask_off;                      // shared-memory byte offset of the stage ring's validity words
 };
+constexpr int W_STAGE_MASK_BYTES = SB * N_IN * 4;    // one 32-lane word per bar and field
 
 // Two-level van Herk / Gil-Werman for LONG windows (p > W_SMEM_MAX), entirely in shared memory.
 // The one-level form (Ext) keeps p + 1 slots per array: the raw values of the current block of p bars, turned in place into
@@ -116,6 +126,17 @@ struct Ext2 {
         if (bars_padded >= p) fetch(0, seg_len(0));          // segment 0 of block 0: first needed when block 1 begins
     }
     __device__ __forceinline__ void finish() { if (pending) { mbar_wait(bar, phase); pending = false; } }   // never exit under a copy
+    // Null-aware variant: `a` starts past every bar and becomes the first bar walked with high AND low valid (the validity
+    // words fold explicit starts in).  A re-read raw row holds the intake's benign 1.0 under a null, not the -inf / +inf the
+    // walked bar got.  No such row reaches a valid output:
+    //  - rows before `a` are masked below, as in the plain kernel.  Every row segment_end() re-reads is older than the bar
+    //    being walked, so `a` is final for it;
+    //  - WILLR / MIDPRICE / Donchian: a symbol flagged in high or low has all-null lines, and an unflagged one has leading
+    //    nulls only, so every row from `a` on is valid in both fields;
+    //  - KDJ: a re-read row enters only the suffixes of bars whose window holds it, and fastk is null on every bar whose last
+    //    k rows hold a null high or low (UnitKdj::step_nulls).
+    // The checkpoints and the prefix extremes come from the walked bars, never from re-read rows.
+    __device__ __forceinline__ void seen(int t, bool hl) { if (hl && t < a) a = t; }
     __device__ __forceinline__ void step(double h, double l, double &hn, double &ln) {
         ph = dmax(ph, h);
         pl = dmin(pl, l);
@@ -171,10 +192,22 @@ struct Ext2 {
     }
 };
 
+__device__ __forceinline__ void seen(Ext &, int, bool) {}                   // (the one-level arrays hold walked bars only)
+__device__ __forceinline__ void seen(Ext2 &e, int t, bool hl) { e.seen(t, hl); }
+
 struct WCtx {
     size_t pos;        // element offset of (this lane, current bar)
     int a, n_bars;     // this lane's first valid bar; bars of the panel
+    size_t mpos;       // null-aware variant: block * bars_padded + bar (ballot words)
+    unsigned flags;    // null-aware variant: this lane's symbol flags
 };
+
+// null-aware variant: value (NaN when null) + the warp's validity word of this bar; called by all 32 lanes together
+__device__ __forceinline__ void emitw(const WCtx &X, double *out, uint32_t *ovm, double v, bool ok) {
+    const unsigned m = __ballot_sync(FULL, ok);
+    stg(out + X.pos, ok ? v : qnan());
+    if ((threadIdx.x & 31) == 0) ovm[X.mpos] = m;
+}
 
 // ---- KDJ(k, sk, sd) ---------------------------------------------------------------------------------------------------------
 template <class EXT, bool PIPED>
@@ -223,6 +256,45 @@ struct UnitKdj {
         stg(U.out[0] + X.pos, ok_);
         stg(U.out[1] + X.pos, od);
         stg(U.out[2] + X.pos, oj);
+    }
+    // ---- null-aware bar: Role5::step_nulls.  vb bit f = field f of this lane is valid at bar t.  polars' rolling max / min
+    // are positional with a full window (fastk null unless close is valid and the last k rows are valid in high and in low);
+    // the two calc_sma passes skip null inputs.  Flags do not kill KDJ.
+    int run_h, run_l, nfk, nsk;
+    uint32_t *ovm[3];
+    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+        const bool vc = vb & F_C, vh = vb & F_H, vl = vb & F_L;
+        seen(ek, t, vh && vl);
+        double hn, ln;
+        ek.step(vh ? h : ninf(), vl ? l : pinf(), hn, ln);
+        run_h = vh ? min(run_h + 1, 1 << 30) : 0;        // rows since the last null, separately for high and low
+        run_l = vl ? min(run_l + 1, 1 << 30) : 0;
+        const bool vfk = vc && run_h >= U.w && run_l >= U.w;
+        bool okk = false, okd = false;
+        double sk = 0.0, sd = 0.0;
+        if (vfk) {
+            const double num = (c - ln) * 100.0, den = hn - ln;
+            const double fk = (den == 0.0) ? num * copysign(pinf(), den) : num / den;
+            const int j1 = nfk++;
+            const double oldf = fr.swap(fk);
+            s_k += fk;
+            if (j1 >= U.sk) s_k -= oldf;
+            if (j1 >= U.sk - 1) {
+                sk = s_k * U.inv_sk;
+                okk = true;
+                const int j2 = nsk++;
+                const double olds = sr.swap(sk);
+                s_d += sk;
+                if (j2 >= U.sd) s_d -= olds;
+                if (j2 >= U.sd - 1) {
+                    sd = s_d * U.inv_sd;
+                    okd = true;
+                }
+            }
+        }
+        emitw(X, U.out[0], ovm[0], sk, okk);
+        emitw(X, U.out[1], ovm[1], sd, okd);
+        emitw(X, U.out[2], ovm[2], 3.0 * sk - 2.0 * sd, okd);
     }
     __device__ __forceinline__ void finish() { ek.finish(); }
     // ---- software-pipelined steady bar (Role5::pipe of the suite kernel): A = window extremes of bar t, B = fastk's division
@@ -301,6 +373,30 @@ struct UnitWmd {
         if (U.out[2]) stg(U.out[2] + X.pos, in ? hn : nn);                                // Donchian upper / lower (D3)
         if (U.out[3]) stg(U.out[3] + X.pos, in ? ln : nn);
     }
+    // ---- null-aware bar: Role6::step_nulls.  The window advances on every bar; a bar without both high and low enters it as
+    // -inf / +inf.  willr is all-null for a symbol flagged in close, high or low, and otherwise valid where close, high and
+    // low are, after p - 1 earlier bars with high and low valid; midprice and the Donchian lines are all-null for a symbol
+    // flagged in high or low, and otherwise valid where high and low are.
+    int n_valid;
+    uint32_t *ovm[4];
+    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+        const bool in = (vb & F_H) && (vb & F_L);
+        seen(ew, t, in);
+        double hn, ln;
+        ew.step(in ? h : ninf(), in ? l : pinf(), hn, ln);
+        if (U.out[0]) {                                   // willr momentum.rs:630-662
+            const bool ok = !(X.flags & (F_C | F_H | F_L)) && in && (vb & F_C) && n_valid >= U.w - 1;
+            const double diff = hn - ln;
+            const bool z = diff == 0.0;
+            const double q = -100.0 * (hn - c) / (z ? 1.0 : diff);
+            emitw(X, U.out[0], ovm[0], z ? 0.0 : q, ok);
+        }
+        const bool v = in && !(X.flags & (F_H | F_L));
+        if (U.out[1]) emitw(X, U.out[1], ovm[1], (hn + ln) / 2.0, v);                   // midprice overlap.rs:401
+        if (U.out[2]) emitw(X, U.out[2], ovm[2], hn, v);                                // Donchian upper / lower (D3)
+        if (U.out[3]) emitw(X, U.out[3], ovm[3], ln, v);
+        n_valid += in ? 1 : 0;
+    }
     __device__ __forceinline__ void finish() { ew.finish(); }
     // ---- software-pipelined steady bar (Role6::pipe): A = window extremes, midprice and the Donchian lines of bar t,
     // B = willr's division of bar t-1
@@ -350,19 +446,38 @@ struct UnitAtr {
         stg(U.out[0] + X.pos, (ok && live) ? atr.y : qnan());
         pc = c;
     }
+    // ---- null-aware bar: Role3::step_nulls.  calc_trange's close.shift(1) is positional: the true range is valid where high
+    // and low are valid and the previous ROW's close is; calc_ema counts valid true ranges only.  Flags do not kill ATR.
+    int n_tr;
+    bool pcv;
+    uint32_t *ovm[1];
+    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+        const bool vtr = t >= 1 && (vb & F_H) && (vb & F_L) && pcv;
+        const double tr = rs_max(rs_max(h - l, fabs(h - pc)), fabs(l - pc));             // volatility.rs:77
+        const bool ok = atr.step<false>(tr, vtr ? n_tr : -1, U.ep, U.alpha);
+        emitw(X, U.out[0], ovm[0], atr.y, ok);
+        n_tr += vtr ? 1 : 0;
+        pc = c;
+        pcv = vb & F_C;
+    }
     __device__ __forceinline__ void finish() {}
     static constexpr int DEPTH = 0;
     template <int M>
     __device__ __forceinline__ void pipe(const WCtx &, double, double, double) {}
 };
 
-template <class UNIT>
+// (NULLS: stage st's validity words are at byte A.mask_off + st * W_STAGE_MASK_BYTES of the shared memory)
+template <bool NULLS, class UNIT>
 __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUnit &U_, uint32_t stage, uint32_t full, int *cnt,
                                          int n_units, int block, int lane, int a) {
     R.take(U_);
     const int sym = block * SYM + lane;
     const int src_lane = (sym < A.n_symbols) ? lane : 0;   // lanes past the last symbol follow lane 0 (no slow-path divisions)
     WCtx X{(size_t)block * A.bars_padded * SYM + lane, a, A.n_bars};
+    if constexpr (NULLS) {
+        X.mpos = (size_t)block * A.bars_padded;
+        X.flags = A.symflags[(sym < A.n_symbols) ? sym : block * SYM];
+    }
     int amax = a;
 #pragma unroll
     for (int d = 16; d >= 1; d >>= 1) amax = max(amax, __shfl_xor_sync(FULL, amax, d));
@@ -390,7 +505,24 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
         else mbar_wait(full + st * 8, (it / ns) & 1);
         const uint32_t sp = st * W_STAGE_BYTES + src_lane * 8;
         const int t0 = it * SB;
-        if (t0 >= steady_from && t0 + SB <= A.n_bars) {
+        if constexpr (NULLS) {
+            // (no software pipelining, no fast stages; bars past the panel's end leave the state as it is)
+            const uint32_t mp = stage + (uint32_t)A.mask_off + st * W_STAGE_MASK_BYTES;
+#pragma unroll 1
+            for (int b = 0; b < SB; ++b) {
+                if (t0 + b < A.n_bars) {
+                    const uint32_t q = sp + b * (SYM * 8);
+                    uint4 mw;
+                    asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
+                                 : "=r"(mw.x), "=r"(mw.y), "=r"(mw.z), "=r"(mw.w) : "r"(mp + b * 16));
+                    // (a ragged block's spare lanes follow lane 0's validity too)
+                    const unsigned vb = ((mw.x >> src_lane) & 1u) | (((mw.y >> src_lane) & 1u) << 1) | (((mw.z >> src_lane) & 1u) << 2);
+                    R.step_nulls(X, t0 + b, lds(q), lds(q + 1 * SB * SYM * 8), lds(q + 2 * SB * SYM * 8), vb);
+                }
+                X.pos += SYM;
+                X.mpos += 1;
+            }
+        } else if (t0 >= steady_from && t0 + SB <= A.n_bars) {
             int b = 0;
             if constexpr (DEPTH > 0) {
                 for (; fill < DEPTH; ++fill, ++b) {        // prime: stage A alone, then A + B
@@ -426,12 +558,15 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
                 atomicExch(&cnt[st], 0);
                 const int nx = it + ns;
                 if (nx < n_iter) {
-                    mbar_expect_tx(full + st * 8, (uint32_t)W_STAGE_BYTES);
+                    mbar_expect_tx(full + st * 8, (uint32_t)W_STAGE_BYTES + (NULLS ? W_STAGE_MASK_BYTES : 0));
                     const size_t off = base + (size_t)nx * SB * SYM;
 #pragma unroll
                     for (int f = 0; f < W_FIELDS; ++f)
                         tma_load_1d(stage + st * W_STAGE_BYTES + f * SB * SYM * 8, A.in[f] + off, (uint32_t)(SB * SYM * sizeof(double)),
                                     full + st * 8);
+                    if constexpr (NULLS)
+                        tma_load_1d(stage + (uint32_t)A.mask_off + st * W_STAGE_MASK_BYTES, A.vmask + (base / SYM + (size_t)nx * SB) * N_IN,
+                                    W_STAGE_MASK_BYTES, full + st * 8);
                 }
             }
         }
@@ -442,8 +577,9 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
 
 // grid = n_blocks * n_groups, blockDim = 32 * (the largest group's units); CTA (b, g): warp i = unit i of group g.
 // Two builds: <128, 4> for up to four units per CTA (118 registers, nothing spilled: at 96 the pipelined loops spill and
-// the launch is slower, profiles/r02p_window_sweep.txt), <192, 2> for five or six.
-template <int MAXT, int MINB>
+// the launch is slower, profiles/r02p_window_sweep.txt), <192, 2> for five or six.  NULLS: the null-aware variant (blocks
+// with a flagged symbol; A.start unused, the validity words carry the starts).
+template <int MAXT, int MINB, bool NULLS = false>
 __global__ void __launch_bounds__(MAXT, MINB) window_suite_kernel(const __grid_constant__ WinArgs A) {
     uint64_t *full_p = reinterpret_cast<uint64_t *>(smem_dyn + A.ns * W_STAGE_BYTES);
     uint64_t *unit_p = full_p + NS;
@@ -453,7 +589,8 @@ __global__ void __launch_bounds__(MAXT, MINB) window_suite_kernel(const __grid_c
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     // group-major: the CTAs of the heaviest group (group 0) are scheduled first, the lighter groups fill in behind them
     const int g = A.block_major ? (int)(blockIdx.x % (unsigned)A.n_groups) : (int)(blockIdx.x / (unsigned)A.n_blocks);
-    const int block = A.block_major ? (int)(blockIdx.x / (unsigned)A.n_groups) : (int)(blockIdx.x % (unsigned)A.n_blocks);
+    const int bi = A.block_major ? (int)(blockIdx.x / (unsigned)A.n_groups) : (int)(blockIdx.x % (unsigned)A.n_blocks);
+    const int block = A.blist ? A.blist[bi] : bi;
     const int n_units = A.n_units[g];
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -465,18 +602,22 @@ __global__ void __launch_bounds__(MAXT, MINB) window_suite_kernel(const __grid_c
         const int n_iter = A.bars_padded / SB;
         const size_t base = (size_t)block * A.bars_padded * SYM;
         for (int it = 0; it < A.ns && it < n_iter; ++it) {
-            mbar_expect_tx(full + it * 8, (uint32_t)W_STAGE_BYTES);
+            mbar_expect_tx(full + it * 8, (uint32_t)W_STAGE_BYTES + (NULLS ? W_STAGE_MASK_BYTES : 0));
 #pragma unroll
             for (int f = 0; f < W_FIELDS; ++f)
                 tma_load_1d(stage + it * W_STAGE_BYTES + f * SB * SYM * 8, A.in[f] + base + (size_t)it * SB * SYM,
                             (uint32_t)(SB * SYM * sizeof(double)), full + it * 8);
+            if constexpr (NULLS)
+                tma_load_1d(stage + (uint32_t)A.mask_off + it * W_STAGE_MASK_BYTES, A.vmask + ((size_t)block * A.bars_padded + (size_t)it * SB) * N_IN,
+                            W_STAGE_MASK_BYTES, full + it * 8);
         }
     }
     __syncthreads();
     if (warp >= n_units) return;
     const WinUnit &U = A.u[A.first[g] + warp];
+    uint32_t *const *ovm = A.ovm[A.first[g] + warp];
     const int sym = block * SYM + lane;
-    const int a = A.start ? A.start[(sym < A.n_symbols) ? sym : block * SYM] : 0;
+    const int a = (!NULLS && A.start) ? A.start[(sym < A.n_symbols) ? sym : block * SYM] : 0;
     const int src_lane = (sym < A.n_symbols) ? lane : 0;
     const size_t pbase = (size_t)block * A.bars_padded * SYM;
     auto kdj = [&](auto &R) {
@@ -484,33 +625,48 @@ __global__ void __launch_bounds__(MAXT, MINB) window_suite_kernel(const __grid_c
         R.sr.init(rings + U.off_sk, U.sd, lane);
         R.s_k = R.s_d = 0.0;
         R.pNum = R.pDen = R.pFk = 0.0;
+        if constexpr (NULLS) {
+            R.run_h = R.run_l = R.nfk = R.nsk = 0;
+            for (int q = 0; q < 3; ++q) R.ovm[q] = ovm[q];
+        }
         __syncwarp();
-        run_unit(R, A, U, stage, full, cnt, n_units, block, lane, a);
+        run_unit<NULLS>(R, A, U, stage, full, cnt, n_units, block, lane, a);
     };
     auto wmd = [&](auto &R) {
         R.pH = R.pL = R.pC = 0.0;
+        if constexpr (NULLS) {
+            R.n_valid = 0;
+            for (int q = 0; q < 4; ++q) R.ovm[q] = ovm[q];
+        }
         __syncwarp();
-        run_unit(R, A, U, stage, full, cnt, n_units, block, lane, a);
+        run_unit<NULLS>(R, A, U, stage, full, cnt, n_units, block, lane, a);
     };
     auto one = [&](auto &R) { R.init(rings + U.off_h, rings + U.off_l, U.w, lane); };
-    auto two = [&](auto &R) { R.init(rings + U.off_h, unit_p + warp, A.in[1] + pbase, A.in[2] + pbase, U.w, U.seg, a, lane, src_lane, A.bars_padded); };
+    // (NULLS: the first bar with high and low valid is found on the walk, Ext2::seen)
+    auto two = [&](auto &R) { R.init(rings + U.off_h, unit_p + warp, A.in[1] + pbase, A.in[2] + pbase, U.w, U.seg, NULLS ? INT_MAX : a, lane, src_lane, A.bars_padded); };
+    // (the null-aware variant has no software-pipelined path)
     if (U.kind == WK_KDJ) {
         if (U.off_l >= 0) {
-            if (U.piped) { UnitKdj<Ext, true> R; one(R.ek); kdj(R); } else { UnitKdj<Ext, false> R; one(R.ek); kdj(R); }
+            if (!NULLS && U.piped) { UnitKdj<Ext, true> R; one(R.ek); kdj(R); } else { UnitKdj<Ext, false> R; one(R.ek); kdj(R); }
         } else {
-            if (U.piped) { UnitKdj<Ext2, true> R; two(R.ek); kdj(R); } else { UnitKdj<Ext2, false> R; two(R.ek); kdj(R); }
+            if (!NULLS && U.piped) { UnitKdj<Ext2, true> R; two(R.ek); kdj(R); } else { UnitKdj<Ext2, false> R; two(R.ek); kdj(R); }
         }
     } else if (U.kind == WK_WMD) {
         if (U.off_l >= 0) {
-            if (U.piped) { UnitWmd<Ext, true> R; one(R.ew); wmd(R); } else { UnitWmd<Ext, false> R; one(R.ew); wmd(R); }
+            if (!NULLS && U.piped) { UnitWmd<Ext, true> R; one(R.ew); wmd(R); } else { UnitWmd<Ext, false> R; one(R.ew); wmd(R); }
         } else {
-            if (U.piped) { UnitWmd<Ext2, true> R; two(R.ew); wmd(R); } else { UnitWmd<Ext2, false> R; two(R.ew); wmd(R); }
+            if (!NULLS && U.piped) { UnitWmd<Ext2, true> R; two(R.ew); wmd(R); } else { UnitWmd<Ext2, false> R; two(R.ew); wmd(R); }
         }
     } else {
         UnitAtr R;
         R.atr.init();
         R.pc = 0.0;
-        run_unit(R, A, U, stage, full, cnt, n_units, block, lane, a);
+        if constexpr (NULLS) {
+            R.n_tr = 0;
+            R.pcv = false;
+            R.ovm[0] = ovm[0];
+        }
+        run_unit<NULLS>(R, A, U, stage, full, cnt, n_units, block, lane, a);
     }
 }
 

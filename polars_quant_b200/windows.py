@@ -8,7 +8,20 @@ for several windows and one ATR over a close / high / low panel (include/pqb200.
 
 Replaces, per symbol, the reference's STOCH(h, l, c, k, 3, 0, 3, 0) (momentum.py:178-186; KDJ per SURVEY D3), willr
 (momentum.rs:630), midprice (overlap.rs:281), atr (volatility.rs:18) called once per window; every value is bit-identical
-to those calls."""
+to those calls.
+
+Panels with halts, delistings, never-listed symbols or fields listed on different rows (validity bitmaps through
+`panel.set_column(..., validity=)` / `set_columns`) follow the suite's null rules: each line equals, in values and validity,
+what `Panel.compute` gives for the same single period.  A field is flagged at its first null after its own first valid bar.
+- KDJ: fastk is valid where close is and the last k rows are valid in high and in low; slowk / slowd skip nulls; J is valid
+  where D is.  Flags do not void KDJ.
+- WILLR: all-null for a symbol flagged in close, high or low; otherwise valid where close, high and low are, after p - 1
+  earlier bars with high and low valid.
+- MIDPRICE / Donchian: all-null for a symbol flagged in high or low; otherwise valid where high and low are, the expanding
+  window counting only such bars.
+- ATR: the true range needs high, low and the previous row's close; the average counts valid true ranges.  Flags do not
+  void ATR.
+Symbol blocks without a flagged symbol run the plain kernel; the others run its null-aware variant beside it."""
 from __future__ import annotations
 
 import ctypes as C

@@ -190,6 +190,26 @@ def split_columns(table: pa.Table, fields):
     return list(symbols), by_field
 
 
+_extra_engines: dict[tuple[int, int], Engine] = {}      # (device, k) -> the k-th further engine of a device (k >= 1)
+
+
+def _shard_engines(devices) -> list[Engine]:
+    """One engine per entry of `devices`.  A panel run drives its engine's streams and fork / join events (include/pqb200.h:
+    one engine per thread), so shards that share a device must not share an engine: the first occurrence of an ordinal
+    gets `get_engine(d)`, every repeat a further engine of that device, created once and reused by later calls."""
+    seen: dict[int, int] = {}
+    out = []
+    for d in devices:
+        k = seen[d] = seen.get(d, -1) + 1
+        if k == 0:
+            out.append(get_engine(d))
+            continue
+        if (d, k) not in _extra_engines:
+            _extra_engines[(d, k)] = Engine(d)
+        out.append(_extra_engines[(d, k)])
+    return out
+
+
 def _f64(col) -> pa.Array:
     a = col.combine_chunks() if isinstance(col, pa.ChunkedArray) else col
     return a if a.type == pa.float64() else a.cast(pa.float64())
@@ -350,8 +370,10 @@ class WidePanel:
         as ONE Arrow record batch (pqb_suite_run_record_batch: intake pipelined with the GPU pipeline) and the results
         come back as ONE record batch aliasing the pinned result planes (pqb_panel_export_arrow) -- no per-column work in
         Python.  `devices`: GPU ordinals to shard the symbols over (contiguous ranges, one host thread per GPU, no
-        collective -- SURVEY.md 8e); default: this panel's engine only.  `lazy=True` returns a `WideResult` (columns wrapped
-        on demand) instead of the full table."""
+        collective -- SURVEY.md 8e); default: this panel's engine only.  Every shard runs on an engine of its own: an
+        ordinal listed more than once (e.g. `[0, 0]`, several shards on one GPU) gets a further engine of that device per
+        repeat, kept for later calls.  `lazy=True` returns a `WideResult` (columns wrapped on demand) instead of the full
+        table."""
         import time
         tm = self.last_timings = {}
         t_ = time.perf_counter()
@@ -373,7 +395,7 @@ class WidePanel:
         lap("release_previous_panel_ms")
         sym, fld = self._suite_map(symbols, cols)
         lap("column_map_ms")
-        engines = [self.engine or get_engine(0)] if not devices else [get_engine(d) for d in devices]
+        engines = [self.engine or get_engine(0)] if not devices else _shard_engines(devices)
         from .shard import symbol_range
         shards = []
         for g, eng in enumerate(engines):

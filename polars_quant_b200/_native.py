@@ -217,6 +217,19 @@ def lib() -> C.CDLL:
         L.pqb_windows_run.argtypes = [C.c_void_p]
         L.pqb_windows_last_launches.argtypes = [C.c_void_p]
         L.pqb_windows_time.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_float)]
+        L.pqb_windows_live_create.argtypes = [C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]
+        L.pqb_windows_live_destroy.argtypes = [C.c_void_p]
+        L.pqb_windows_live_destroy.restype = None
+        L.pqb_windows_live_bars.argtypes = [C.c_void_p]
+        L.pqb_windows_live_bars.restype = C.c_int64
+        L.pqb_windows_live_state_bytes.argtypes = [C.c_void_p]
+        L.pqb_windows_live_state_bytes.restype = C.c_int64
+        L.pqb_windows_live_push.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
+        for name in ("pqb_windows_live_host_output", "pqb_windows_live_host_validity", "pqb_windows_live_host_voided"):
+            f = getattr(L, name)
+            f.restype = C.c_void_p
+            f.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_windows_live_last_push_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         # candle engine
         L.pqb_candle_params_default.argtypes = [C.POINTER(CandleParams)]
         L.pqb_candle_params_default.restype = None

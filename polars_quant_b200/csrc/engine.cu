@@ -2577,3 +2577,4 @@ extern "C" int pqb_multi_run_host(pqb_multi *m, const pqb_suite_params *params) 
 #include "signals_host.inc"
 #include "info_host.inc"
 #include "live_host.inc"
+#include "windows_live_host.inc"

@@ -84,7 +84,11 @@ constexpr int W_STAGE_MASK_BYTES = SB * N_IN * 4;    // one 32-lane word per bar
 // (100 MB for config 5), which the 28 output streams evicted from L2 -- 21.5 GB of DRAM traffic for 12.5 GB of algorithmic
 // bytes and an L2 / DRAM round trip on every bar's critical path (profiles/r02k_launch_summary.txt).
 // max / min are exact, so the association (segments, checkpoints) does not change a bit of the result.
-struct Ext2 {
+// LIVE (window_live_kernel): a walk may stop at any bar and a later launch resume from the saved object.  Such a walk
+// issues no copy at init -- the rows of segment 0 may not exist yet -- and fetches them on entering block 0's last
+// segment, when all of them have been walked; resume() re-issues the copy a saved walk had in flight.
+template <bool LIVE = false>
+struct Ext2T {
     uint32_t bh, bl, rh, rl, ah, al;   // byte offsets in shared memory (this lane's column; raw: the source lane's)
     uint32_t rdst, bar, phase;         // TMA destination (row 0 of raw high; raw low follows b rows later), this unit's mbarrier
     uint32_t roff, endoff;             // byte offset of slot r + 1 of buf; (len + 1) * 256
@@ -168,7 +172,10 @@ struct Ext2 {
         const int len = seg_len(s);
         roff = SYM * 8;
         endoff = (uint32_t)(len + 1) * (SYM * 8);
-        if (k == 0) return;                                // no previous block yet: buf keeps its sentinels
+        if (k == 0) {                                      // no previous block yet: buf keeps its sentinels
+            if constexpr (LIVE) { if (s == m - 1) fetch(0, seg_len(0)); }
+            return;
+        }
         // suffix extremes of segment s of block k - 1 from its raw rows, on top of the checkpoint of the segments after it
         mbar_wait(bar, phase);
         phase ^= 1;
@@ -190,10 +197,34 @@ struct Ext2 {
         const int s2 = (s + 1 == m) ? 0 : s + 1;
         fetch(t0 + len, seg_len(s2));                      // segments are contiguous in time
     }
+    // LIVE: continue a saved walk.  mbarrier phases and bulk copies end with their launch, so the unit's barrier starts
+    // afresh (phase 0) and the copy the saved walk had in flight -- the rows the next segment_end() reads: segment s + 1 of
+    // block k - 1, or segment 0 of block k from block k's last segment on -- is issued again.  A live walk has such a copy
+    // in flight exactly when k >= 1 or s == m - 1 (the saved `pending` says nothing: finish() cleared it before the save).
+    // Those rows lie 1 .. p - 1 bars before the walk's first bar (the host keeps at least p of them in front of the pushed
+    // rows).  `high` / `low`: the planes' addresses of absolute bar 0.  The caller has put the raw rows' shared memory in
+    // place (generic proxy).
+    __device__ __forceinline__ void resume(uint64_t *mb, const double *high, const double *low) {
+        gh = high; gl = low;
+        bar = smem_u32(mb); phase = 0;
+        if (lane == 0) {
+            mbar_init(mb, 1);
+            fence_mbar_init();
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        }
+        __syncwarp();
+        pending = false;
+        if (k >= 1 || s == m - 1) {
+            const int s2 = (s + 1 == m) ? 0 : s + 1;
+            fetch((s + 1 == m) ? k * p : (k - 1) * p + s2 * b, seg_len(s2));
+        }
+    }
 };
+using Ext2 = Ext2T<false>;
 
 __device__ __forceinline__ void seen(Ext &, int, bool) {}                   // (the one-level arrays hold walked bars only)
-__device__ __forceinline__ void seen(Ext2 &e, int t, bool hl) { e.seen(t, hl); }
+template <bool L>
+__device__ __forceinline__ void seen(Ext2T<L> &e, int t, bool hl) { e.seen(t, hl); }
 
 struct WCtx {
     size_t pos;        // element offset of (this lane, current bar)
@@ -207,6 +238,13 @@ __device__ __forceinline__ void emitw(const WCtx &X, double *out, uint32_t *ovm,
     const unsigned m = __ballot_sync(FULL, ok);
     stg(out + X.pos, ok ? v : qnan());
     if ((threadIdx.x & 31) == 0) ovm[X.mpos] = m;
+}
+// live walks: the prime walk over a history stores nothing (store = 0)
+struct WCtxLive : WCtx {
+    bool store;
+};
+__device__ __forceinline__ void emitw(const WCtxLive &X, double *out, uint32_t *ovm, double v, bool ok) {
+    if (X.store) emitw(static_cast<const WCtx &>(X), out, ovm, v, ok);
 }
 
 // ---- KDJ(k, sk, sd) ---------------------------------------------------------------------------------------------------------
@@ -262,7 +300,8 @@ struct UnitKdj {
     // the two calc_sma passes skip null inputs.  Flags do not kill KDJ.
     int run_h, run_l, nfk, nsk;
     uint32_t *ovm[3];
-    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+    template <class CX>
+    __device__ __forceinline__ void step_nulls(const CX &X, int t, double c, double h, double l, unsigned vb) {
         const bool vc = vb & F_C, vh = vb & F_H, vl = vb & F_L;
         seen(ek, t, vh && vl);
         double hn, ln;
@@ -379,7 +418,8 @@ struct UnitWmd {
     // flagged in high or low, and otherwise valid where high and low are.
     int n_valid;
     uint32_t *ovm[4];
-    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+    template <class CX>
+    __device__ __forceinline__ void step_nulls(const CX &X, int t, double c, double h, double l, unsigned vb) {
         const bool in = (vb & F_H) && (vb & F_L);
         seen(ew, t, in);
         double hn, ln;
@@ -451,7 +491,8 @@ struct UnitAtr {
     int n_tr;
     bool pcv;
     uint32_t *ovm[1];
-    __device__ __forceinline__ void step_nulls(const WCtx &X, int t, double c, double h, double l, unsigned vb) {
+    template <class CX>
+    __device__ __forceinline__ void step_nulls(const CX &X, int t, double c, double h, double l, unsigned vb) {
         const bool vtr = t >= 1 && (vb & F_H) && (vb & F_L) && pcv;
         const double tr = rs_max(rs_max(h - l, fabs(h - pc)), fabs(l - pc));             // volatility.rs:77
         const bool ok = atr.step<false>(tr, vtr ? n_tr : -1, U.ep, U.alpha);
@@ -466,14 +507,30 @@ struct UnitAtr {
     __device__ __forceinline__ void pipe(const WCtx &, double, double, double) {}
 };
 
+// Live window panels (windows_live_host.inc): a walk covers the absolute bars [t_base, A.n_bars).  The input planes are
+// [block][in_stride][32] with the walk's first bar at A.in[f] (row `tail` of each block: the high / low rows before it stay
+// readable for Ext2's re-reads); outputs and validity words are [block][A.bars_padded] from the walk's first bar.  The
+// state of CTA (block, group) is the unit objects (word i of unit warp u, lane l at (u * W_LIVE_UNIT_WORDS + i) * 32 + l)
+// followed by the CTA's ring area.
+struct WinLiveArgs {
+    unsigned long long *state;         // [n_blocks][n_groups][group_words]
+    long long group_words;             // W_MAX_UNITS * W_LIVE_UNIT_WORDS * 32 + ring_bytes / 8
+    int ring_bytes;                    // the largest group's ring area (smem_bytes minus stages and control area)
+    int t_base;                        // absolute index of the walk's first bar
+    int in_stride;                     // rows per symbol block of the input planes
+    int prime;                         // 1: the units start from init() and store nothing; 0: they resume from the state
+    int commit;                        // 1: the walk's end state is written back
+};
+
 // (NULLS: stage st's validity words are at byte A.mask_off + st * W_STAGE_MASK_BYTES of the shared memory)
-template <bool NULLS, class UNIT>
+template <bool NULLS, class UNIT, bool LIVE = false>
 __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUnit &U_, uint32_t stage, uint32_t full, int *cnt,
-                                         int n_units, int block, int lane, int a) {
+                                         int n_units, int block, int lane, int a, const WinLiveArgs *L = nullptr) {
     R.take(U_);
     const int sym = block * SYM + lane;
     const int src_lane = (sym < A.n_symbols) ? lane : 0;   // lanes past the last symbol follow lane 0 (no slow-path divisions)
-    WCtx X{(size_t)block * A.bars_padded * SYM + lane, a, A.n_bars};
+    std::conditional_t<LIVE, WCtxLive, WCtx> X{WCtx{(size_t)block * A.bars_padded * SYM + lane, a, A.n_bars}};
+    if constexpr (LIVE) X.store = !L->prime;
     if constexpr (NULLS) {
         X.mpos = (size_t)block * A.bars_padded;
         X.flags = A.symflags[(sym < A.n_symbols) ? sym : block * SYM];
@@ -484,6 +541,7 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
     const long long steady_from = (long long)amax + A.steady_lead;
     const int n_iter = A.bars_padded / SB;
     const size_t base = (size_t)block * A.bars_padded * SYM;
+    const size_t ibase = LIVE ? (size_t)block * L->in_stride * SYM : base;   // (input planes)
     const int ns = A.ns;
     // software-pipelined steady path: `fill` = primed pipeline stages (warp-uniform); drained before any general bar
     constexpr int DEPTH = UNIT::DEPTH, PIPE_ALL = (1 << (DEPTH + 1)) - 1;
@@ -504,7 +562,7 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
         if (A.relaxed_wait) mbar_wait_relaxed(full + st * 8, (it / ns) & 1);
         else mbar_wait(full + st * 8, (it / ns) & 1);
         const uint32_t sp = st * W_STAGE_BYTES + src_lane * 8;
-        const int t0 = it * SB;
+        const int t0 = (LIVE ? L->t_base : 0) + it * SB;
         if constexpr (NULLS) {
             // (no software pipelining, no fast stages; bars past the panel's end leave the state as it is)
             const uint32_t mp = stage + (uint32_t)A.mask_off + st * W_STAGE_MASK_BYTES;
@@ -559,7 +617,7 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
                 const int nx = it + ns;
                 if (nx < n_iter) {
                     mbar_expect_tx(full + st * 8, (uint32_t)W_STAGE_BYTES + (NULLS ? W_STAGE_MASK_BYTES : 0));
-                    const size_t off = base + (size_t)nx * SB * SYM;
+                    const size_t off = ibase + (size_t)nx * SB * SYM;
 #pragma unroll
                     for (int f = 0; f < W_FIELDS; ++f)
                         tma_load_1d(stage + st * W_STAGE_BYTES + f * SB * SYM * 8, A.in[f] + off, (uint32_t)(SB * SYM * sizeof(double)),
@@ -573,6 +631,41 @@ __device__ __forceinline__ void run_unit(UNIT &R, const WinArgs &A, const WinUni
     }
     if constexpr (DEPTH > 0) { if (fill) drain(); }
     R.finish();
+}
+
+// ---- live walks: unit objects and the CTA's ring area <-> the state buffer ----------------------------------------------------
+static_assert(std::is_trivially_copyable<UnitKdj<Ext, false>>::value && std::is_trivially_copyable<UnitKdj<Ext2T<true>, false>>::value &&
+              std::is_trivially_copyable<UnitWmd<Ext, false>>::value && std::is_trivially_copyable<UnitWmd<Ext2T<true>, false>>::value &&
+              std::is_trivially_copyable<UnitAtr>::value, "a unit object is saved and restored as raw bytes");
+constexpr size_t w_max(size_t a, size_t b) { return a > b ? a : b; }
+constexpr int W_LIVE_UNIT_WORDS = (int)(w_max(w_max(w_max(sizeof(UnitKdj<Ext, false>), sizeof(UnitKdj<Ext2T<true>, false>)),
+                                                   w_max(sizeof(UnitWmd<Ext, false>), sizeof(UnitWmd<Ext2T<true>, false>))),
+                                             sizeof(UnitAtr)) + 7) / 8;
+
+// a unit object <-> its words (lane-interleaved: a warp moves 256 contiguous bytes per word)
+template <bool LOAD, class UNIT>
+__device__ __forceinline__ void win_live_unit(UNIT &R, unsigned long long *uw, int lane) {
+    static_assert(sizeof(UNIT) % 8 == 0, "unit objects are saved in 8-byte words");
+    constexpr int W = (int)(sizeof(UNIT) / 8);
+    unsigned long long w[W];
+    if (!LOAD) __builtin_memcpy(w, &R, sizeof(UNIT));
+#pragma unroll
+    for (int i = 0; i < W; ++i) {
+        if (LOAD) w[i] = uw[(size_t)i * SYM + lane];
+        else uw[(size_t)i * SYM + lane] = w[i];
+    }
+    if (LOAD) __builtin_memcpy(&R, w, sizeof(UNIT));
+}
+
+// the CTA's ring area <-> the state buffer: the unit warps' threads move 16-byte pieces
+template <bool LOAD>
+__device__ __forceinline__ void win_live_rings(double *rings, unsigned long long *grp, int ring_bytes, int n_threads) {
+    uint4 *g = reinterpret_cast<uint4 *>(grp + (size_t)W_MAX_UNITS * W_LIVE_UNIT_WORDS * SYM);
+    uint4 *s = reinterpret_cast<uint4 *>(rings);
+    for (int u = threadIdx.x; u < ring_bytes / 16; u += n_threads) {
+        if (LOAD) s[u] = g[u];
+        else g[u] = s[u];
+    }
 }
 
 // grid = n_blocks * n_groups, blockDim = 32 * (the largest group's units); CTA (b, g): warp i = unit i of group g.
@@ -667,6 +760,93 @@ __global__ void __launch_bounds__(MAXT, MINB) window_suite_kernel(const __grid_c
             R.ovm[0] = ovm[0];
         }
         run_unit<NULLS>(R, A, U, stage, full, cnt, n_units, block, lane, a);
+    }
+}
+
+// live window panels: the null-aware walk of every symbol block, resumable (WinLiveArgs).  The stage ring is the null-aware
+// kernel's; the input planes are [block][L.in_stride][32].  (Its own kernel rather than a template flag of the one above:
+// moving that kernel's body into a shared function changes the register assignment of the plain builds.)
+template <int MAXT, int MINB>
+__global__ void __launch_bounds__(MAXT, MINB) window_live_kernel(const __grid_constant__ WinArgs A, const __grid_constant__ WinLiveArgs Lv) {
+    const WinLiveArgs *L = &Lv;
+    uint64_t *full_p = reinterpret_cast<uint64_t *>(smem_dyn + A.ns * W_STAGE_BYTES);
+    uint64_t *unit_p = full_p + NS;
+    int *cnt = reinterpret_cast<int *>(unit_p + W_MAX_UNITS);
+    double *rings = reinterpret_cast<double *>(smem_dyn + A.ns * W_STAGE_BYTES + W_CTRL_BYTES);
+    const uint32_t stage = smem_u32(smem_dyn), full = smem_u32(full_p);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int g = A.block_major ? (int)(blockIdx.x % (unsigned)A.n_groups) : (int)(blockIdx.x / (unsigned)A.n_blocks);
+    const int block = A.block_major ? (int)(blockIdx.x / (unsigned)A.n_groups) : (int)(blockIdx.x % (unsigned)A.n_blocks);
+    const int n_units = A.n_units[g];
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int s = 0; s < NS; ++s) {
+            mbar_init(&full_p[s], 1);
+            cnt[s] = 0;
+        }
+        fence_mbar_init();
+        const int n_iter = A.bars_padded / SB;
+        const size_t ibase = (size_t)block * L->in_stride * SYM;
+        for (int it = 0; it < A.ns && it < n_iter; ++it) {
+            mbar_expect_tx(full + it * 8, (uint32_t)(W_STAGE_BYTES + W_STAGE_MASK_BYTES));
+#pragma unroll
+            for (int f = 0; f < W_FIELDS; ++f)
+                tma_load_1d(stage + it * W_STAGE_BYTES + f * SB * SYM * 8, A.in[f] + ibase + (size_t)it * SB * SYM,
+                            (uint32_t)(SB * SYM * sizeof(double)), full + it * 8);
+            tma_load_1d(stage + (uint32_t)A.mask_off + it * W_STAGE_MASK_BYTES, A.vmask + ((size_t)block * A.bars_padded + (size_t)it * SB) * N_IN,
+                        W_STAGE_MASK_BYTES, full + it * 8);
+        }
+    }
+    __syncthreads();
+    if (warp >= n_units) return;
+    const WinUnit &U = A.u[A.first[g] + warp];
+    uint32_t *const *ovm = A.ovm[A.first[g] + warp];
+    const int sym = block * SYM + lane;
+    const int src_lane = (sym < A.n_symbols) ? lane : 0;
+    const int a = 0;                                         // (the validity words carry the starts)
+    // ---- live walk: every unit object starts from init() (prime) or from the state, and goes back there on commit ----
+    unsigned long long *grp = L->state + ((size_t)block * A.n_groups + g) * L->group_words;
+    unsigned long long *uw = grp + (size_t)warp * W_LIVE_UNIT_WORDS * SYM;
+    if (!L->prime) win_live_rings<true>(rings, grp, L->ring_bytes, n_units * 32);
+    roles_sync(n_units);                                 // every piece of the ring area is in place
+    // the high / low planes' addresses of absolute bar 0 (Ext2's re-reads index them by absolute bar)
+    const double *gh = A.in[1] + ((ptrdiff_t)block * L->in_stride - L->t_base) * SYM;
+    const double *gl = A.in[2] + ((ptrdiff_t)block * L->in_stride - L->t_base) * SYM;
+    auto go = [&](auto &R, auto &&init, auto &&resume) {
+        if (L->prime) init();
+        else {
+            win_live_unit<true>(R, uw, lane);
+            resume();
+        }
+        for (int q = 0; q < (int)(sizeof(R.ovm) / sizeof(R.ovm[0])); ++q) R.ovm[q] = ovm[q];
+        __syncwarp();
+        run_unit<true, std::remove_reference_t<decltype(R)>, true>(R, A, U, stage, full, cnt, n_units, block, lane, a, L);
+        if (L->commit) {
+            win_live_unit<false>(R, uw, lane);
+            roles_sync(n_units);                         // no unit warp touches the ring area any more
+            win_live_rings<false>(rings, grp, L->ring_bytes, n_units * 32);
+        }
+    };
+    auto kdj0 = [&](auto &R) {
+        R.fr.init(rings + U.off_fk, U.sk, lane);
+        R.sr.init(rings + U.off_sk, U.sd, lane);
+        R.s_k = R.s_d = 0.0;
+        R.pNum = R.pDen = R.pFk = 0.0;
+        R.run_h = R.run_l = R.nfk = R.nsk = 0;
+    };
+    auto wmd0 = [&](auto &R) { R.pH = R.pL = R.pC = 0.0; R.n_valid = 0; };
+    // (bars_padded 0: no copy at init, Ext2T<true>)
+    auto two = [&](auto &E) { E.init(rings + U.off_h, unit_p + warp, gh, gl, U.w, U.seg, INT_MAX, lane, src_lane, 0); };
+    auto nothing = [] {};
+    if (U.kind == WK_KDJ) {
+        if (U.off_l >= 0) { UnitKdj<Ext, false> R; go(R, [&] { R.ek.init(rings + U.off_h, rings + U.off_l, U.w, lane); kdj0(R); }, nothing); }
+        else { UnitKdj<Ext2T<true>, false> R; go(R, [&] { two(R.ek); kdj0(R); }, [&] { R.ek.resume(unit_p + warp, gh, gl); }); }
+    } else if (U.kind == WK_WMD) {
+        if (U.off_l >= 0) { UnitWmd<Ext, false> R; go(R, [&] { R.ew.init(rings + U.off_h, rings + U.off_l, U.w, lane); wmd0(R); }, nothing); }
+        else { UnitWmd<Ext2T<true>, false> R; go(R, [&] { two(R.ew); wmd0(R); }, [&] { R.ew.resume(unit_p + warp, gh, gl); }); }
+    } else {
+        UnitAtr R;
+        go(R, [&] { R.atr.init(); R.pc = 0.0; R.n_tr = 0; R.pcv = false; }, nothing);
     }
 }
 

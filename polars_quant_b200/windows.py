@@ -21,10 +21,20 @@ what `Panel.compute` gives for the same single period.  A field is flagged at it
   window counting only such bars.
 - ATR: the true range needs high, low and the previous row's close; the average counts valid true ranges.  Flags do not
   void ATR.
-Symbol blocks without a flagged symbol run the plain kernel; the others run its null-aware variant beside it."""
+Symbol blocks without a flagged symbol run the plain kernel; the others run its null-aware variant beside it.
+
+Live window panels: `wp.live(max_push_bars=64)` primes a `WindowLive` from the panel's device inputs; each
+`push(close, high, low, valid=None, commit=True)` takes k new bars of every symbol and returns {name: (values [S, k],
+validity [S, k])}, bit-identical to the last k rows of `compute()` over the concatenated history with the same validity.
+Pushes may carry any validity pattern, under the null rules above applied per push: a first null after a field's first
+valid bar flags it, and a new flag can turn a symbol's whole WILLR (close / high / low) or MIDPRICE / Donchian (high / low)
+column null, history included -- `voided` names those columns after each push ({name: symbol indices}).  commit=False
+previews a bar: the rows come back, the state stays.  The live panel keeps no reference to the window panel."""
 from __future__ import annotations
 
 import ctypes as C
+
+import numpy as np
 
 from . import _native as N
 from .panel import Engine, Panel, get_engine
@@ -89,3 +99,95 @@ class WindowPanel:
         ms = C.c_float()
         N.check(N.lib().pqb_windows_time(self._h, warmup, iters, C.byref(ms)))
         return ms.value / iters, N.lib().pqb_windows_last_launches(self._h)
+
+    def live(self, max_push_bars: int = 64) -> "WindowLive":
+        """A live window panel primed from this panel's device inputs (compute / upload / fill_synthetic first)."""
+        return WindowLive(self, max_push_bars)
+
+
+class WindowLive:
+    """Append bars to a many-window panel (include/pqb200.h "live window panels"); see the module docstring."""
+    FIELDS = ("close", "high", "low")
+
+    def __init__(self, wp: WindowPanel, max_push_bars: int = 64):
+        self.n_symbols = wp.n_symbols
+        self.max_push_bars = int(max_push_bars)
+        self.names = wp.names()                     # {slot: name}
+        self.voided = {}                            # (the last push's; a new dict per push)
+        self.engine = wp.engine                     # (the native engine must outlive the live panel)
+        self._h = C.c_void_p()
+        N.check(N.lib().pqb_windows_live_create(wp._h, C.c_int64(max_push_bars), C.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            N.lib().pqb_windows_live_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def bars(self) -> int:
+        """History bars + committed bars."""
+        return int(N.lib().pqb_windows_live_bars(self._h))
+
+    @property
+    def state_bytes(self) -> int:
+        return int(N.lib().pqb_windows_live_state_bytes(self._h))
+
+    def last_push_ms(self) -> float:
+        """Device milliseconds of the last push (CUDA events from the pack of the new rows to the unpack of the results)."""
+        ms = C.c_float()
+        N.check(N.lib().pqb_windows_live_last_push_ms(self._h, C.byref(ms)))
+        return ms.value
+
+    def _rows(self, name, a, k, dtype=np.float64):
+        if a is None:
+            raise ValueError("%s is required" % name)
+        a = np.asarray(a, dtype=dtype)
+        if a.ndim == 1:
+            a = a[None, :]
+        if a.ndim != 2 or a.shape[1] != self.n_symbols:
+            raise ValueError("%s has shape %r: expected [k, %d] or [%d]" % (name, a.shape, self.n_symbols, self.n_symbols))
+        if k is not None and a.shape[0] != k:
+            raise ValueError("%s has %d bars, close has %d" % (name, a.shape[0], k))
+        return np.ascontiguousarray(a)
+
+    def push(self, close, high, low, valid=None, commit: bool = True):
+        """k new bars: close / high / low float64 [k, n_symbols] (or [n_symbols] for one bar); `valid` None (all valid), one
+        bool array for every field, or a dict {field: bool array} of the same shape.  Returns {name: (values, validity)} of
+        shape [n_symbols, k] and sets `voided`: {name: indices of the symbols whose earlier rows of that line this push
+        turned null} (a preview's too)."""
+        c = self._rows("close", close, None)
+        k = c.shape[0]
+        if k > self.max_push_bars:
+            raise ValueError("%d bars in one push; this live window panel takes at most %d" % (k, self.max_push_bars))
+        vals = {"close": c, "high": self._rows("high", high, k), "low": self._rows("low", low, k)}
+        masks = {}
+        if valid is not None:
+            per = valid if isinstance(valid, dict) else {f: valid for f in self.FIELDS}
+            for f, m in per.items():
+                if f not in self.FIELDS:
+                    raise ValueError("unknown field %r in valid (close, high, low)" % (f,))
+                masks[f] = np.packbits(self._rows("valid", m, k, bool), axis=1, bitorder="little")
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        N.check(N.lib().pqb_windows_live_push(self._h, C.c_int64(k), *(ptr(vals[f]) for f in self.FIELDS),
+                                              *(ptr(masks.get(f)) for f in self.FIELDS), 1 if commit else 0))
+        vb = (self.n_symbols + 7) // 8
+        res, voided = {}, {}
+        for slot, name in self.names.items():
+            vp = N.lib().pqb_windows_live_host_output(self._h, slot)
+            bp = N.lib().pqb_windows_live_host_validity(self._h, slot)
+            v = np.ctypeslib.as_array((C.c_double * (k * self.n_symbols)).from_address(vp)).reshape(k, self.n_symbols)
+            b = np.ctypeslib.as_array((C.c_uint8 * (k * vb)).from_address(bp)).reshape(k, vb)
+            ok = np.unpackbits(b, axis=1, bitorder="little")[:, :self.n_symbols].astype(bool)
+            res[name] = (v.T.copy(), ok.T.copy())
+            w = np.ctypeslib.as_array((C.c_uint8 * vb).from_address(N.lib().pqb_windows_live_host_voided(self._h, slot)))
+            syms = np.flatnonzero(np.unpackbits(w, bitorder="little")[:self.n_symbols])
+            if len(syms):
+                voided[name] = syms
+        self.voided = voided
+        return res

@@ -862,32 +862,18 @@ struct Built {
     int steady_b;              // a.steady_lead of the benchmark groups alone (their own null-aware launch next to optional groups)
 };
 
-static bool split_launch_enabled() {
-    const char *s = getenv("PQB_SPLIT_LAUNCH");           // (0: one general launch for everything -- measurement knob)
-    return !s || atoi(s) != 0;
-}
-
 // panels of up to this many symbol blocks run the small-panel variant of the full suite (nine pipelined role warps, two
-// CTAs per SM); PQB_SMALL_BLOCKS overrides (tuning)
+// CTAs per SM)
 // CTAs per tail block: as many as keeps the tail launch at about half a CTA per SM (measured, profiles/r03a_compact_tail.txt:
 // 9 tail blocks -> one role per CTA, 24 -> three roles per CTA; more tail CTAs than that cost more than they spread)
 static int tail_parts_compact(const pqb_engine *e, int64_t n_tail) {
-    static const int forced = getenv("PQB_TAIL_PARTS") ? std::max(1, std::min((int)N_ROLES_X, atoi(getenv("PQB_TAIL_PARTS")))) : 0;
-    if (forced) return forced;
     const int64_t by_budget = (e->sm_count * 55ll / 100) / std::max<int64_t>(n_tail, 1);
     return (int)std::max<int64_t>(2, std::min<int64_t>(N_ROLES_X, by_budget));
 }
-static bool tail_compact() {
-    static const bool v = !getenv("PQB_TAIL_COMPACT") || atoi(getenv("PQB_TAIL_COMPACT")) != 0;
-    return v;
-}
 static int64_t small_max_blocks(const pqb_engine *e) {
-    static const char *ev = getenv("PQB_SMALL_BLOCKS");
-    if (ev) return atoll(ev);
     // one whole-block CTA per SM + up to sm_count / 5 blocks beyond as compact tail CTAs (beyond that the plain kernel with two
     // CTAs on some SMs is as fast: 196 blocks 1.61 against 1.59 ms)
-    if (tail_compact()) return e->sm_count + e->sm_count / 5;
-    return e->sm_count + e->sm_count / N_ROLES_X;
+    return e->sm_count + e->sm_count / 5;
 }
 
 // shared-memory ring layout of one launch: offsets of every enabled group's rings / van Herk arrays and the dynamic
@@ -1179,7 +1165,7 @@ static int build_args(const pqb_panel *p, const pqb_suite_params *sp, Built *out
     // benchmark groups next to optional groups run as two launches, each with its own layout (launch_suite): what has to
     // fit is each half, not their union (e.g. WILLR(250) + MIDPRICE(250) next to DONCHIAN(250))
     const unsigned gb = A.gmask & (unsigned)G_ALL, go = A.gmask & ~(unsigned)G_ALL;
-    if (gb && go && !A.vmask && split_launch_enabled()) {
+    if (gb && go && !A.vmask) {
         for (unsigned part : {gb, go}) {
             SuiteArgs t = A;
             t.gmask = part;
@@ -1248,18 +1234,16 @@ static void deal_base_slots(SuiteArgs &A) {
     }
     struct Cut { int role; unsigned half; };
     const Cut cuts[] = {{6, (unsigned)(G_MIDPRICE)}, {4, (unsigned)G_AD}, {0, (unsigned)(G_MACD | G_SMA)}, {3, (unsigned)G_NATR}};
-    const char *ds = getenv("PQB_DEAL_SLOTS");
-    if (!ds || atoi(ds) != 0)
-        for (const Cut &c : cuts) {
-            if (n >= N_ROLES) break;
-            if (c.role == 6 && !A.mid_own) continue;
-            for (int w = 0; w < n; ++w) {
-                if (A.slot_role[w] != c.role) continue;
-                const unsigned a = A.slot_mask[w] & c.half, b = A.slot_mask[w] & ~c.half;
-                if (a && b) { A.slot_mask[w] = b; A.slot_role[n] = c.role; A.slot_mask[n] = a; ++n; }
-                break;
-            }
+    for (const Cut &c : cuts) {
+        if (n >= N_ROLES) break;
+        if (c.role == 6 && !A.mid_own) continue;
+        for (int w = 0; w < n; ++w) {
+            if (A.slot_role[w] != c.role) continue;
+            const unsigned a = A.slot_mask[w] & c.half, b = A.slot_mask[w] & ~c.half;
+            if (a && b) { A.slot_mask[w] = b; A.slot_role[n] = c.role; A.slot_mask[n] = a; ++n; }
+            break;
         }
+    }
     // role -> slot code: 3 * role, + 1 for the half without the cut groups, + 2 for the cut half
     for (int w = 0; w < n; ++w) {
         const int role = A.slot_role[w];
@@ -1277,16 +1261,11 @@ static void deal_base_slots(SuiteArgs &A) {
 // the null-aware variant of a launch's arguments: per-bar validity words in, per-bar validity words out, starts folded
 // into the masks
 // fully valid stages of a null-aware launch run the plain steady step (suite_kernel.cuh run_role): only for launches of the 21 suite
-// outputs -- the optional outputs report validity per bar through emitv, with null rules of their own (PQB_NULLS_FAST=0: never)
+// outputs -- the optional outputs report validity per bar through emitv, with null rules of their own
 static int nulls_fast_ok(const SuiteArgs &a) {
-    static const bool on = !getenv("PQB_NULLS_FAST") || atoi(getenv("PQB_NULLS_FAST")) != 0;
-    if (!on || (a.gmask & ~(unsigned)G_ALL) || a.don_fold) return 0;
+    if ((a.gmask & ~(unsigned)G_ALL) || a.don_fold) return 0;
     for (int k = PQB_N_SUITE_OUTPUTS; k < PQB_N_OUTPUTS; ++k) if (a.out[k]) return 0;
     return 1;
-}
-static bool nulls_fulls() {              // PQB_NULLS_FULLS=0: the general null-aware kernel also for the full suite
-    static const bool on = !getenv("PQB_NULLS_FULLS") || atoi(getenv("PQB_NULLS_FULLS")) != 0;
-    return on;
 }
 static SuiteArgs null_variant(const pqb_panel *p, SuiteArgs a) {
     a.nulls_fast = nulls_fast_ok(a);
@@ -1297,13 +1276,7 @@ static SuiteArgs null_variant(const pqb_panel *p, SuiteArgs a) {
     return a;
 }
 
-// tuning: PQB_FULLS_SMEM = dynamic shared memory requested for the full-suite kernel (more than it needs = fewer CTAs per SM)
-static int fulls_smem(int need) {
-    static const char *ev = getenv("PQB_FULLS_SMEM");
-    return ev ? std::max(need, atoi(ev)) : need;
-}
-
-// One thread that sleeps ~`ns` nanoseconds on the main stream (PQB_COMPACT_DELAY_US, default 40): the null-aware CTAs of a symbol
+// One thread that sleeps ~`ns` nanoseconds on the main stream (kCompactDelayUs): the null-aware CTAs of a symbol
 // compaction are then resident -- one per SM, each asking for the SM's whole shared memory so that no plain CTA moves in beside
 // it -- before the plain grid fills the rest of the GPU.  Measured with a timeline build (globaltimer stamps, profiles/
 // r03_halted_symbols.txt): without it they only start when the first plain wave ends (2.0 ms in); sharing an SM with a plain CTA
@@ -1316,11 +1289,7 @@ __global__ void delay_kernel(unsigned ns) {
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     } while (t - t0 < ns);
 }
-
-static bool force_base() {
-    static const bool v = getenv("PQB_FORCE_BASE") && atoi(getenv("PQB_FORCE_BASE")) != 0;
-    return v;
-}
+static constexpr unsigned kCompactDelayUs = 40;
 
 // Launches the suite over symbol blocks [b0, b0+nb) (+ NaN fills + validity bitmaps of those symbols).
 static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb, cudaEvent_t ev_after_fused,
@@ -1347,17 +1316,12 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         // CTA shape of a launch with few role warps per block (partial suites, optional groups): field-sized stages and the CTA
         // width with the fewest waves -- see the comment at the partial-suite launch below
         auto shape_few_warps = [&](const void *kernel, SuiteArgs &x, int n_slots, int &threads, int &smem) {
-            static const bool slim = !getenv("PQB_BASE_SLIM") || atoi(getenv("PQB_BASE_SLIM")) != 0;
-            static const int warps = getenv("PQB_BASE_WARPS") ? atoi(getenv("PQB_BASE_WARPS")) : 0;
-            static const int min_smem = getenv("PQB_BASE_SMEM") ? atoi(getenv("PQB_BASE_SMEM")) : 0;
             int top = 0;
             for (int f = 0; f < N_IN; ++f) if (x.fields >> f & 1) top = f + 1;
-            x.stage_stride = slim ? top * SB * SYM * 8 : STAGE_BYTES;
-            smem = std::max(x.smem_bytes - NS * (STAGE_BYTES - x.stage_stride), min_smem);
+            x.stage_stride = top * SB * SYM * 8;
+            smem = x.smem_bytes - NS * (STAGE_BYTES - x.stage_stride);
             threads = CTA_THREADS;
-            int occ = 0;
-            if (warps > 0) threads = 32 * std::min(N_ROLES + 1, std::max(warps, n_slots + 1));
-            else if (x.split_from < 0 && nb > 3ll * e->sm_count) {          // (up to three blocks per SM the eight-warp CTA is one wave already)
+            if (x.split_from < 0 && nb > 3ll * e->sm_count) {               // (up to three blocks per SM the eight-warp CTA is one wave already)
                 int64_t best = INT64_MAX;
                 for (int W = N_ROLES + 1; W > n_slots; --W) {
                     // (warp w runs on SM sub-partition w % 4: the producer -- the last warp, polling its mbarriers -- must not share
@@ -1367,21 +1331,15 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
                     int k = 0;
                     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k, kernel, 32 * W, (size_t)smem) != cudaSuccess || k <= 0) continue;
                     const int64_t waves = (nb + (int64_t)k * e->sm_count - 1) / ((int64_t)k * e->sm_count);
-                    if (waves < best) { best = waves; threads = 32 * W; occ = k; }
+                    if (waves < best) { best = waves; threads = 32 * W; }
                 }
             }
             // Two-warp CTAs (one slot + the producer): the role warps of the resident CTAs all sat on two of the four SM sub-partitions (ncu, EMA
             // alone: one scheduler 95 % busy, the next 9 %) -- warp slots go to CTAs in pairs, so CTA j of an SM (blocks sm_count apart) swaps
             // role and producer warp when (j / 2) is odd (suite_kernel.cuh base_rot).  EMA alone 0.81 -> 0.72 ms (0.85 of peak), RSI 1.86 -> 1.31.
-            // Wider CTAs: every rotation measured was slower (BBANDS, four warps: 1.68 -> 1.80 - 1.98 ms).  PQB_BASE_ROT=0: off
-            static const int rot = getenv("PQB_BASE_ROT") ? atoi(getenv("PQB_BASE_ROT")) : 1;
-            x.base_rot = (rot && x.split_from < 0 && threads == 64) ? e->sm_count : 0;
+            // Wider CTAs: every rotation measured was slower (BBANDS, four warps: 1.68 -> 1.80 - 1.98 ms).
+            x.base_rot = (x.split_from < 0 && threads == 64) ? e->sm_count : 0;
             x.base_rot_pair = 1;
-            static const bool print_occ = getenv("PQB_PRINT_OCC") != nullptr;
-            if (print_occ) {
-                if (!occ) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, (size_t)smem);
-                fprintf(stderr, "[pqb] few-warp launch: %d slots, %d threads, %d B smem -> %d CTAs per SM, %lld blocks\n", n_slots, threads, smem, occ, (long long)nb);
-            }
         };
 #if defined(PQB_DEBUG_CLOCKS) || defined(PQB_DEBUG_SMID)      // tuning builds: per-role busy cycles of the first block (costs ~18% on config 4) / the SM of every CTA
         if (!g_dbg) { CU(cudaMalloc(&g_dbg, 4096 * sizeof(unsigned long long))); CU(cudaMemset(g_dbg, 0xff, 4096 * sizeof(unsigned long long))); }
@@ -1400,40 +1358,26 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         // 222 blocks split 1.41 ms, unsplit 0.84 ms).
         a.split_from = -1;
         unsigned grid = (unsigned)nb;
-        const char *ts = getenv("PQB_TAIL_SPLIT");
-        const bool tail_ok = !ts || atoi(ts) != 0;
-        const char *ps = getenv("PQB_PIPELINE");
-        const bool pipe_ok = !ps || atoi(ps) != 0;
         // the small-panel variant: nine role warps (two CTAs of 320 threads fit an SM)
-        const bool small = fulls && pipe_ok && !a.vmask && a.mid_own && nb <= small_max_blocks(e);
+        const bool small = fulls && !a.vmask && a.mid_own && nb <= small_max_blocks(e);
         // a launch of optional groups only: the general kernel with its seven warps dealt as slots (suite_kernel.cuh)
-        const char *ws = getenv("PQB_WIDE");
-        const bool wide = !a.vmask && a.gmask && !(a.gmask & (unsigned)G_ALL) && (!ws || atoi(ws) != 0);
+        const bool wide = !a.vmask && a.gmask && !(a.gmask & (unsigned)G_ALL);
         const int nr = small ? N_ROLES_X : wide ? N_SLOTS_W : N_ROLES;
-        int parts = nr;                                       // in-grid tail CTAs per split block (default: one role each)
-        if (const char *tp = getenv("PQB_TAIL_PARTS")) if (!tail_compact()) parts = std::max(1, std::min(nr, atoi(tp)));
-        a.split_parts = parts;
+        a.split_parts = nr;                                   // in-grid tail CTAs per split block: one role each
         a.split_compact = 0;
-        if (tail_ok && nb > e->sm_count && nb <= e->sm_count + e->sm_count / nr && !(small && tail_compact())) {
+        if (nb > e->sm_count && nb <= e->sm_count + e->sm_count / nr && !small) {
             a.split_from = e->sm_count;
-            grid = (unsigned)(e->sm_count + (nb - e->sm_count) * parts);
+            grid = (unsigned)(e->sm_count + (nb - e->sm_count) * nr);
         }
-        // tuning: PQB_SPLIT_ALL=<parts> splits EVERY block of a launch between one and two CTAs per SM into that many CTAs
-        static const int split_all = getenv("PQB_SPLIT_ALL") ? atoi(getenv("PQB_SPLIT_ALL")) : 0;
-        if (split_all > 1 && fulls && !small && nb > e->sm_count + e->sm_count / nr && nb < 2ll * e->sm_count) {
-            a.split_from = 0;
-            a.split_parts = std::min(nr, split_all);
-            grid = (unsigned)(nb * a.split_parts);
-        }
-        if (a.vmask && fulls && a.nulls_fast && nulls_fulls()) suite_fused_kernel<true, true><<<grid, CTA_THREADS, a.smem_bytes, e->stream>>>(a);
+        if (a.vmask && fulls && a.nulls_fast) suite_fused_kernel<true, true><<<grid, CTA_THREADS, a.smem_bytes, e->stream>>>(a);
         else if (a.vmask) suite_fused_kernel<false, true><<<grid, CTA_THREADS, a.smem_bytes, e->stream>>>(a);
         // small panels (about one CTA per SM) are bound by the length of each role's dependent FP64 chain per bar, not by
         // issue slots or HBM: they run the variant whose division-heavy roles (BBANDS, RSI, STOCH) are software-pipelined
         // over bars (suite_kernel.cuh "software-pipelined steady bar"); large panels are throughput-bound and run the
         // plain one (the pipelined loops execute more instructions)
-        else if (small && tail_compact() && tail_ok && nb > e->sm_count) {
+        else if (small && nb > e->sm_count) {
             // one whole-block CTA per SM; the blocks beyond run beside them as COMPACT tail CTAs (a launch of its own on a
-            // second stream: `parts` CTAs per block, each 32 * (roles per CTA + 1) threads with its own producer and ring),
+            // second stream: `cp` CTAs per block, each 32 * (roles per CTA + 1) threads with its own producer and ring),
             // so a tail CTA holds 4 warps of registers instead of 10 and the block scheduler can put two of them next to a
             // whole-block CTA -- no SM walks two whole blocks
             const int cp = tail_parts_compact(e, nb - e->sm_count);
@@ -1452,12 +1396,7 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         }
         else if (small)
             suite_fused_kernel<true, false, false, true><<<grid, CTA_THREADS_X, a.smem_bytes, e->stream>>>(a);
-        else if (fulls && force_base()) {                   // tuning: the partial-suite kernel (seven warps, pipelined roles) on the full suite
-            deal_base_slots(a);
-            a.stage_stride = STAGE_BYTES;
-            suite_fused_kernel<false, false, true><<<grid, CTA_THREADS, a.smem_bytes, e->stream>>>(a);
-        }
-        else if (fulls) suite_fused_kernel<true, false><<<grid, CTA_THREADS, fulls_smem(a.smem_bytes), e->stream>>>(a);
+        else if (fulls) suite_fused_kernel<true, false><<<grid, CTA_THREADS, a.smem_bytes, e->stream>>>(a);
         else if (!(a.gmask & ~(unsigned)G_ALL) && !fastk) {
             deal_base_slots(a);
             // A partial suite has few role warps per block, so an eight-warp CTA (three per SM by registers) leaves a large panel
@@ -1465,8 +1404,6 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             // (profiles/r05_partial_suite_cta_shapes.txt): the TMA stages hold only the fields this launch reads (close alone: 2 KB
             // per stage instead of 8), and the CTA is launched with W warps, n_slots + 1 <= W <= 8 -- the W with the fewest waves,
             // the widest such (fewer co-resident walks are faster walks).  EMA 1.24 -> 0.81 ms, RSI 2.36 -> 1.85, BBANDS 2.10 -> 1.68.
-            // tuning: PQB_BASE_SLIM=0 full-size stages, PQB_BASE_WARPS=W fixes the width (8 = as before), PQB_BASE_SMEM = dynamic
-            // shared memory to ask for at least, PQB_PRINT_OCC=1 prints the choice
             int threads, smem;
             shape_few_warps((const void *)suite_fused_kernel<false, false, true>, a, a.n_roles, threads, smem);
             suite_fused_kernel<false, false, true><<<grid, threads, smem, e->stream>>>(a);
@@ -1498,20 +1435,19 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         // The benchmark suite's null-aware kernel (<FULLS, NULLS> with fast stages) walks a block with a few halted symbols about as fast
         // as the plain kernel does, so flagged blocks simply run through it, beside the plain launch: no gather, no write-back, no
         // scattered stores (50,000 x 5,040 with 5 % halted symbols: 22.8 ms compacted).  Symbol compaction stays for the launches that
-        // kernel does not serve (partial suites).  PQB_NULLS_PREFER_DISPATCH=0: compact whenever the panel is prepared for it.
-        static const bool prefer_dispatch = !getenv("PQB_NULLS_PREFER_DISPATCH") || atoi(getenv("PQB_NULLS_PREFER_DISPATCH")) != 0;
-        bool fast_suite = prefer_dispatch && full.a.gmask == (unsigned)G_ALL && nulls_fast_ok(full.a) && nulls_fulls();
+        // kernel does not serve (partial suites).
+        bool fast_suite = full.a.gmask == (unsigned)G_ALL && nulls_fast_ok(full.a);
         for (int k = 0; k < PQB_N_SUITE_OUTPUTS; ++k) fast_suite &= full.a.out[k] != nullptr;
         // ... on a panel of several waves with more than a handful of flagged symbols.  A null-aware CTA that shares its SM with plain CTAs
         // in the latency regime walks 1.6x slower (8,192 x 5,040 with 83 halted symbols: 3.0 ms dispatched, 2.2 ms compacted onto SMs of
         // their own), and up to ~64 flagged symbols the gather / write-back is cheaper than a slower block per symbol (20,000 x 5,040:
         // 20 halted 5.5 ms compacted / 5.8 dispatched, 200 halted 6.2 / 5.2)
         // (beyond 1,024 flagged symbols compaction stores straight into the symbols' lanes -- scattered 8-byte stores, ~0.15 ms per compacted
-        // block: there the dispatch wins on a small panel too; PQB_NULLS_DISPATCH_SMALL_FROM = that count)
-        static const int small_from = getenv("PQB_NULLS_DISPATCH_SMALL_FROM") ? atoi(getenv("PQB_NULLS_DISPATCH_SMALL_FROM")) : 1024;
+        // block: there the dispatch wins on a small panel too)
+        constexpr int kCompactDirectFrom = 1024;
         // ... and whenever four blocks out of five hold a flagged symbol anyway (8,192 x 5,040 with 409 halted symbols, one per block or more:
         // 3.7 ms compacted, 2.25 ms with every block in the null-aware kernel)
-        fast_suite = fast_suite && ((nb > 3ll * e->sm_count && p->n_x > 64) || p->n_x > small_from || n_null * 5 >= nb * 4);
+        fast_suite = fast_suite && ((nb > 3ll * e->sm_count && p->n_x > 64) || p->n_x > kCompactDirectFrom || n_null * 5 >= nb * 4);
         did_compact = p->compact && n_null && !go && b0 == 0 && nb == p->n_blocks && !fast_suite;
         if (did_compact) {
             // ---- symbol compaction: flagged symbols -> blocks of their own (null-aware kernel, second stream) while the plain
@@ -1533,8 +1469,7 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             // while the plain kernel runs, and a write-back pass (~3.6 us per symbol) puts the lanes in place.  DIRECT (many): the
             // null-aware kernel runs AFTER the plain one on the same stream and stores straight into the symbols' own lanes
             // (SuiteArgs::symmap), overwriting what the plain kernel left there -- no overlap, but no write-back either.
-            static const int direct_from = getenv("PQB_COMPACT_DIRECT_FROM") ? atoi(getenv("PQB_COMPACT_DIRECT_FROM")) : 1024;
-            const bool direct = p->n_x > direct_from;
+            const bool direct = p->n_x > kCompactDirectFrom;
             SuiteArgs an = full.a;
             an.nulls_fast = nulls_fast_ok(full.a);
             an.start = nullptr;
@@ -1547,18 +1482,14 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             an.split_from = -1; an.split_parts = N_ROLES; an.split_compact = 0; an.dbg = nullptr;
             if (!an.smem_bytes && (rc = layout_rings(an, p))) return rc;
             derive_roles(an);
-            // (exclusive: with the whole shared memory of an SM requested, no plain CTA can move in beside a null-aware CTA)
-            static const int exclusive = getenv("PQB_COMPACT_EXCLUSIVE") ? atoi(getenv("PQB_COMPACT_EXCLUSIVE")) : 1;
-            static const int split0 = getenv("PQB_COMPACT_SPLIT0") ? atoi(getenv("PQB_COMPACT_SPLIT0")) : 1;
-            bool fulls_n = an.gmask == (unsigned)G_ALL && an.nulls_fast && nulls_fulls();
+            // (with the whole shared memory of an SM requested, no plain CTA can move in beside a null-aware CTA)
+            bool fulls_n = an.gmask == (unsigned)G_ALL && an.nulls_fast;
             for (int k = 0; k < PQB_N_SUITE_OUTPUTS; ++k) fulls_n &= an.out[k] != nullptr;
             auto launch_null = [&](cudaStream_t st) {
                 if (fulls_n)                // (exactly the benchmark suite: the compile-time-specialised null-aware kernel)
-                    suite_fused_kernel<true, true><<<(unsigned)n_xb, CTA_THREADS, exclusive ? kMaxSmem : an.smem_bytes, st>>>(an);
-                else if (split0 && exclusive)    // (the variant with SMA / EMA / TEMA / MACD over two warps: 288 threads, one CTA per SM)
+                    suite_fused_kernel<true, true><<<(unsigned)n_xb, CTA_THREADS, kMaxSmem, st>>>(an);
+                else                        // (the variant with SMA / EMA / TEMA / MACD over two warps: 288 threads, one CTA per SM)
                     suite_fused_kernel<false, true, false, true><<<(unsigned)n_xb, CTA_THREADS + 32, kMaxSmem, st>>>(an);
-                else
-                    suite_fused_kernel<false, true><<<(unsigned)n_xb, CTA_THREADS, exclusive ? kMaxSmem : an.smem_bytes, st>>>(an);
                 ++n_launch;
                 return cudaGetLastError();
             };
@@ -1570,13 +1501,9 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             } else {
                 CU(launch_null(e->aux));
                 CU(cudaEventRecord(e->ev_join, e->aux));
-                static const int order = getenv("PQB_COMPACT_ORDER") ? atoi(getenv("PQB_COMPACT_ORDER")) : 0;
-                if (order == 0) {
-                    CU(cudaStreamWaitEvent(e->stream, e->ev_pre, 0));
-                    static const int delay_us = getenv("PQB_COMPACT_DELAY_US") ? atoi(getenv("PQB_COMPACT_DELAY_US")) : 40;
-                    if (delay_us > 0) { delay_kernel<<<1, 32, 0, e->stream>>>((unsigned)delay_us * 1000u); CU(cudaGetLastError()); }
-                }
-                if (order == 2) CU(cudaStreamWaitEvent(e->stream, e->ev_join, 0));  // (tuning: no overlap at all)
+                CU(cudaStreamWaitEvent(e->stream, e->ev_pre, 0));
+                delay_kernel<<<1, 32, 0, e->stream>>>(kCompactDelayUs * 1000u);
+                CU(cudaGetLastError());
                 if ((rc = launch_one(ap, nullptr, nb))) return rc;
                 CU(cudaStreamWaitEvent(e->stream, e->ev_join, 0));
                 CompactArgs Sc{};
@@ -1604,14 +1531,11 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             plain_list = p->d_blist + b0;
             null_list = p->d_blist + p->n_blocks + b0;
         }
-        // per-block dispatch with both kinds of blocks: the null-aware launch (the longer walk) goes first, on the second stream,
-        // and the plain launch runs beside it (8,192 x 5,040 with one halted symbol: 1.6 + 1.9 ms back to back -> side by side)
-        static const bool side_by_side = !getenv("PQB_NULLS_CONCURRENT") || atoi(getenv("PQB_NULLS_CONCURRENT")) != 0;
         // the flagged blocks.  Next to optional groups the benchmark groups keep a null-aware launch of their own -- the
         // specialised kernel with fast stages when all 21 suite outputs are bound, as without optional groups -- and the optional
         // groups, whose null rules have no fast stages, walk the same blocks through the general null-aware kernel.
         auto launch_null = [&]() -> int {
-            if (gb && go && split_launch_enabled()) {
+            if (gb && go) {
                 SuiteArgs ab = null_variant(p, full.a), ao = ab;
                 ab.gmask = gb;
                 ab.steady_lead = full.steady_b;
@@ -1627,7 +1551,9 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
             return launch_one(an, null_list, n_null);
         };
         bool null_done = false;
-        if (!did_compact && n_null && n_null < nb && side_by_side) {
+        // per-block dispatch with both kinds of blocks: the null-aware launch (the longer walk) goes first, on the second stream,
+        // and the plain launch runs beside it (8,192 x 5,040 with one halted symbol: 1.6 + 1.9 ms back to back -> side by side)
+        if (!did_compact && n_null && n_null < nb) {
             CU(cudaEventRecord(e->ev_fork, e->stream));       // (after the block lists' copies)
             CU(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
             std::swap(e->stream, e->side);                    // (a null-aware launch_one() touches e->stream only)
@@ -1638,7 +1564,7 @@ static int launch_suite(pqb_panel *p, const Built &full, int64_t b0, int64_t nb,
         }
         if (!did_compact && n_null < nb) {                    // the plain blocks
             const int64_t nl = nb - n_null;
-            if (gb && go && split_launch_enabled()) {
+            if (gb && go) {
                 SuiteArgs ab = full.a, ao = full.a;
                 ab.gmask = gb;
                 ao.gmask = go;

@@ -259,6 +259,18 @@ def lib() -> C.CDLL:
                               C.c_double, C.c_void_p]
         L.pqb_price.argtypes = [C.c_void_p, C.c_int, C.POINTER(Col), C.POINTER(Col), C.POINTER(Col), C.POINTER(Col),
                                 C.POINTER(OutCol)]
+        # live candle panels
+        L.pqb_candles_live_create.argtypes = [C.c_void_p, C.POINTER(CandleParams), C.c_int64, C.POINTER(C.c_void_p)]
+        L.pqb_candles_live_destroy.argtypes = [C.c_void_p]
+        L.pqb_candles_live_destroy.restype = None
+        L.pqb_candles_live_bars.argtypes = [C.c_void_p]
+        L.pqb_candles_live_bars.restype = C.c_int64
+        L.pqb_candles_live_push.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 8 + [C.c_int]
+        for name in ("pqb_candles_live_host_pattern", "pqb_candles_live_host_price", "pqb_candles_live_host_price_validity"):
+            f = getattr(L, name)
+            f.restype = C.c_void_p
+            f.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_candles_live_last_push_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
         # live panels
         L.pqb_live_create.argtypes = [C.c_void_p, C.POINTER(SuiteParams), C.c_uint64, C.c_int64, C.POINTER(C.c_void_p)]
         L.pqb_live_destroy.argtypes = [C.c_void_p]

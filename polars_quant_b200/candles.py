@@ -110,6 +110,100 @@ class CandlePanel:
         N.check(N.lib().pqb_candles_time(self._h, C.byref(p), warmup, iters, C.byref(ms)))
         return float(ms.value)
 
+    def live(self, params: N.CandleParams | None = None, max_push_bars: int = 64) -> "CandleLive":
+        """A live candle panel primed from this panel's device inputs (run_host / fill_synthetic / fill_random_walk first).
+        `params` (default: this panel's masks) chooses the outputs of the pushes, independently of this panel's planes."""
+        return CandleLive(self, params, max_push_bars)
+
+
+class CandleLive:
+    """Append bars to a candle panel (include/pqb200.h "live candle panels").  Each push of k bars returns those k rows of
+    every enabled pattern and price output, bit-identical to the last k rows of CandlePanel.run_host over the concatenated
+    history.  Patterns and BOP refuse nulls (PqbError, PQB_ERR_NULLS); the price transforms propagate them.  commit=False
+    previews a bar: the rows come back, the state stays.  The live panel keeps no reference to the candle panel."""
+    FIELDS = ("open", "high", "low", "close")
+
+    def __init__(self, cp: CandlePanel, params: N.CandleParams | None = None, max_push_bars: int = 64):
+        self.params = params or default_params(cp.patterns_mask, cp.prices_mask)
+        self.n_symbols = cp.n_symbols
+        self.max_push_bars = int(max_push_bars)
+        self.patterns = [k for k in range(N.N_PATTERNS) if self.params.patterns >> k & 1]
+        self.prices = [k for k in range(N.N_PRICES) if self.params.prices >> k & 1]
+        self.engine = cp.engine                     # (the native engine must outlive the live panel)
+        self._h = C.c_void_p()
+        N.check(N.lib().pqb_candles_live_create(cp._h, C.byref(self.params), C.c_int64(max_push_bars), C.byref(self._h)))
+        names = pattern_names()
+        self._pattern_names = {k: names[k] for k in self.patterns}
+
+    def close(self):
+        if self._h:
+            N.lib().pqb_candles_live_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def bars(self) -> int:
+        """History bars + committed bars."""
+        return int(N.lib().pqb_candles_live_bars(self._h))
+
+    def last_push_ms(self) -> float:
+        """Device milliseconds of the last push (CUDA events from the copy of the new rows to the device to the end of the
+        walk)."""
+        ms = C.c_float()
+        N.check(N.lib().pqb_candles_live_last_push_ms(self._h, C.byref(ms)))
+        return ms.value
+
+    def _rows(self, name, a, k, dtype=np.float64):
+        a = np.asarray(a, dtype=dtype)
+        if a.ndim == 1:
+            a = a[None, :]
+        if a.ndim != 2 or a.shape[1] != self.n_symbols:
+            raise ValueError("%s has shape %r: expected [k, %d] or [%d]" % (name, a.shape, self.n_symbols, self.n_symbols))
+        if k is not None and a.shape[0] != k:
+            raise ValueError("%s has %d bars, expected %d" % (name, a.shape[0], k))
+        return np.ascontiguousarray(a)
+
+    def push(self, open=None, high=None, low=None, close=None, valid=None, commit: bool = True):
+        """k new bars: each field float64 [k, n_symbols] (or [n_symbols] for one bar); a field no enabled output reads may
+        be None.  `valid` None (all valid), one bool array for every field, or a dict {field: bool array} of the same shape.
+        Returns ({pattern name: Int32 [n_symbols, k]}, {price name: (values, validity) [n_symbols, k]}) -- the orientation
+        of CandlePanel.pattern() / .price()."""
+        vals, k = {}, None
+        for f, a in zip(self.FIELDS, (open, high, low, close)):
+            if a is not None:
+                vals[f] = self._rows(f, a, k)
+                k = vals[f].shape[0]
+        if k is None:
+            raise ValueError("no field given")
+        if k > self.max_push_bars:
+            raise ValueError("%d bars in one push; this live candle panel takes at most %d" % (k, self.max_push_bars))
+        masks = {}
+        if valid is not None:
+            per = valid if isinstance(valid, dict) else {f: valid for f in self.FIELDS}
+            for f, m in per.items():
+                if f not in self.FIELDS:
+                    raise ValueError("unknown field %r in valid (open, high, low, close)" % (f,))
+                masks[f] = np.packbits(self._rows("valid", m, k, bool), axis=1, bitorder="little")
+        ptr = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        N.check(N.lib().pqb_candles_live_push(self._h, C.c_int64(k), *(ptr(vals.get(f)) for f in self.FIELDS),
+                                              *(ptr(masks.get(f)) for f in self.FIELDS), 1 if commit else 0))
+        n, vb = self.n_symbols, (self.n_symbols + 7) // 8
+        pats, prices = {}, {}
+        for p in self.patterns:
+            a = np.ctypeslib.as_array((C.c_int32 * (k * n)).from_address(N.lib().pqb_candles_live_host_pattern(self._h, p)))
+            pats[self._pattern_names[p]] = a.reshape(k, n).T.copy()
+        for q in self.prices:
+            v = np.ctypeslib.as_array((C.c_double * (k * n)).from_address(N.lib().pqb_candles_live_host_price(self._h, q)))
+            b = np.ctypeslib.as_array((C.c_uint8 * (k * vb)).from_address(N.lib().pqb_candles_live_host_price_validity(self._h, q)))
+            ok = np.unpackbits(b.reshape(k, vb), axis=1, bitorder="little")[:, :n].astype(bool)
+            prices[N.PRICE_NAMES[q]] = (v.reshape(k, n).T.copy(), ok.T.copy())
+        return pats, prices
+
 
 def _col(a):
     a = np.ascontiguousarray(a, dtype=np.float64)

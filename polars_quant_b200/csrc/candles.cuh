@@ -171,12 +171,7 @@ __global__ void __launch_bounds__(CANDLE_TILE, 3) candle_kernel(const __grid_con
                 if ((tid & 31) == 0 && A.vprice[k]) A.vprice[k][(size_t)s * A.words_per_row + w] = m;
             }
         };
-        emit(0, (o0 + h0 + l0 + c0) * 0.25, ko && kh && kl && kc);          // avgprice price.rs:10
-        emit(1, (h0 + l0) * 0.5, kh && kl);                                 // medprice :35
-        emit(2, (h0 + l0 + c0) / 3.0, kh && kl && kc);                      // typprice :55
-        emit(3, (h0 + l0 + 2.0 * c0) / 4.0, kh && kl && kc);                // wclprice :75
-        const double diff = h0 - l0;                                        // bop momentum.rs:113-135
-        emit(4, (diff == 0.0) ? 0.0 : (c0 - o0) / ((diff == 0.0) ? 1.0 : diff), ko && kh && kl && kc);
+#include "candle_prices.inc"
     }
     if (!ALL && pmask == 0) return;
 
@@ -187,162 +182,130 @@ __global__ void __launch_bounds__(CANDLE_TILE, 3) candle_kernel(const __grid_con
     const double o3 = so[q - 3], h3 = sh[q - 3], l3 = sl[q - 3], c3 = sc[q - 3];
     const double o4 = so[q - 4], h4 = sh[q - 4], l4 = sl[q - 4], c4 = sc[q - 4];
     const unsigned f1 = sf[q - 1], f2 = sf[q - 2], f3 = sf[q - 3], f4 = sf[q - 4];
-    const double b0 = fabs(o0 - c0), b1 = fabs(o1 - c1), b2 = fabs(o2 - c2);
-    const double us0 = h0 - fmax(o0, c0), ls0 = fmin(o0, c0) - l0;
-    const double hl0 = h0 + l0;
-    const double near_t = 0.01 * hl0 * 0.5, equal_t = 0.001 * hl0 * 0.5;     // near / equal use the CURRENT bar's range
-#define HAS(f, m) (((f) & (m)) == (m))
-#define NEAR(a, b) (fabs((a) - (b)) < near_t)
-#define EQUAL(a, b) (fabs((a) - (b)) < equal_t)
-    const bool bull0 = f0 & CF_BULL, bear0 = f0 & CF_BEAR, bull1 = f1 & CF_BULL, bear1 = f1 & CF_BEAR;
-    const bool bull2 = f2 & CF_BULL, bear2 = f2 & CF_BEAR;
-    const bool lbull0 = HAS(f0, CF_BULL | CF_LONG), lbear0 = HAS(f0, CF_BEAR | CF_LONG);
-    const bool lbull1 = HAS(f1, CF_BULL | CF_LONG), lbear1 = HAS(f1, CF_BEAR | CF_LONG);
-    const bool lbull2 = HAS(f2, CF_BULL | CF_LONG), lbear2 = HAS(f2, CF_BEAR | CF_LONG);
-    const bool lbull4 = HAS(f4, CF_BULL | CF_LONG), lbear4 = HAS(f4, CF_BEAR | CF_LONG);
-    const bool doji0 = f0 & CF_DOJI, doji1 = f1 & CF_DOJI, short0 = f0 & CF_SHORT, short1 = f1 & CF_SHORT;
-    const bool maru0 = HAS(f0, CF_LONG | CF_VSUS | CF_VSDS), maru1 = HAS(f1, CF_LONG | CF_VSUS | CF_VSDS);
-    const bool lb1 = i >= 1, lb2 = i >= 2, lb3 = i >= 3, lb4 = i >= 4;
     const size_t at = row + i;
     int32_t *const pbase = A.pat[0] + at;
     const size_t pstride = A.pat_stride;
+#define HAS(f, m) (((f) & (m)) == (m))
+#define NEAR(a, b) (fabs((a) - (b)) < near_t)
+#define EQUAL(a, b) (fabs((a) - (b)) < equal_t)
     // `up` -> +100, else `dn` -> -100, else 0.  (A warp-voted early-out on the flag preconditions was measured:
     // on random-walk data almost every 32-bar warp has a lane that passes, and the votes cost more than they save.)
 #define EMIT(id, up, dn)                                                                   \
     if (ALL || (pmask >> (id) & 1)) {                                                      \
         if (live) st_i32(ALL ? pbase + (size_t)(id) * pstride : A.pat[id] + at, (up) ? 100 : ((dn) ? -100 : 0)); \
     }
-    const bool bear3 = f3 & CF_BEAR, bull3 = f3 & CF_BULL, short2 = f2 & CF_SHORT, short3 = f3 & CF_SHORT, doji2 = f2 & CF_DOJI;
-    const bool long0 = f0 & CF_LONG, long1 = f1 & CF_LONG, long2 = f2 & CF_LONG, long4 = f4 & CF_LONG;
-
-    EMIT(P_cdl2crows, false,                                      // pattern.rs:10 (can never fire:
-         lb2 && lbull2 && bear1 && o1 > c2 && bear0 && (o0 > o1 && o0 < c1) && (c0 > o2 && c0 < c2))   //  o0 > o1 && o0 < c1 with c1 < o1)
-    EMIT(P_cdl3blackcrows, false,                               // :43
-         lb2 && lbear2 && lbear1 && lbear0 && (o1 < o2 && o1 > c2) && (o0 < o1 && o0 > c1) && (c1 < c2 && c0 < c1))
-    EMIT(P_cdl3inside,                                                               // :76
-         lb2 && lbear2 && bull1 && c1 < o2 && o1 > c2 && bull0 && c0 > o2,
-         lb2 && lbull2 && bear1 && o1 < c2 && c1 > o2 && bear0 && c0 < o2)
-    EMIT(P_cdl3linestrike,   // :114
-         lb3 && bear3 && bear2 && bear1 && c2 < c3 && c1 < c2 && o2 > c3 && o2 < o3 && o1 > c2 && o1 < o2 && bull0 && o0 < c1 && c0 > o3,
-         lb3 && bull3 && bull2 && bull1 && c2 > c3 && c1 > c2 && o2 < c3 && o2 > o3 && o1 < c2 && o1 > o2 && bear0 && o0 > c1 && c0 < o3)
-    EMIT(P_cdl3outside,           // :160
-         lb2 && bear2 && bull1 && o1 <= c2 && c1 >= o2 && bull0 && c0 > c1,
-         lb2 && bull2 && bear1 && o1 >= c2 && c1 <= o2 && bear0 && c0 < c1)
-    EMIT(P_cdl3starsinsouth,           // :194
-         lb2 && lbear2 && (f2 & CF_LDS) && bear1 && l1 > l2 && c1 > c2 && bear0 && short0 && h0 < h1 && l0 > l1, false)
-    EMIT(P_cdl3whitesoldiers,                                   // :234
-         lb2 && lbull2 && lbull1 && lbull0 && (o1 > o2 && o1 <= c2) && (o0 > o1 && o0 <= c1) && (c1 > c2 && c0 > c1), false)
-    EMIT(P_cdlabandonedbaby,                                                // :268
-         lb2 && lbear2 && doji1 && h1 < l2 && bull0 && l0 > h1,
-         lb2 && lbull2 && doji1 && l1 > h2 && bear0 && h0 < l1)
-    EMIT(P_cdladvanceblock, false,                                // :309
-         lb2 && lbull2 && bull1 && bull0 && (o1 > o2 && o1 <= c2) && (o0 > o1 && o0 <= c1) && (c1 > c2 && c0 > c1) && b0 < b1)
-    EMIT(P_cdlbelthold, lbull0 && (f0 & CF_VSDS), lbear0 && (f0 & CF_VSUS))                       // :345
-    EMIT(P_cdlbreakaway,                                                             // :373
-         lb4 && lbear4 && bear3 && o3 < c4 && c2 < c3 && bull0 && c0 > o3 && c0 < c4,
-         lb4 && lbull4 && bull3 && o3 > c4 && c2 > c3 && bear0 && c0 < o3 && c0 > c4)
-    EMIT(P_cdlclosingmarubozu, lbull0 && (f0 & CF_VSUS), lbear0 && (f0 & CF_VSDS))                // :414
-    EMIT(P_cdlconcealbabyswall,
-         lb3 && HAS(f3, CF_BEAR | CF_LONG | CF_VSUS | CF_VSDS) && HAS(f2, CF_BEAR | CF_LONG | CF_VSUS | CF_VSDS) && c2 < c3 &&
-             bear1 && h1 > c2 && lbear0 && o0 > h1 && c0 < l2, false)
-    EMIT(P_cdlcounterattack,                                                // :487
-         lb1 && lbear1 && lbull0 && NEAR(c0, c1), lb1 && lbull1 && lbear0 && NEAR(c0, c1))
-    EMIT(P_cdldarkcloudcover, false,                                       // :519
-         lb1 && lbull1 && bear0 && o0 > c1 && c0 < (c1 - (b1 * A.pen[PEN_DARKCLOUDCOVER])) && c0 > o1)
-    EMIT(P_cdldoji, doji0, false)                                                                 // :553
-    EMIT(P_cdldojistar,                                                     // :578
-         lb1 && lbear1 && doji0 && ((o0 + c0) / 2.0) < c1, lb1 && lbull1 && doji0 && ((o0 + c0) / 2.0) > c1)
-    EMIT(P_cdldragonflydoji, HAS(f0, CF_DOJI | CF_LDS | CF_VSUS), false)                          // :610
-    EMIT(P_cdlengulfing,                            // :635
-         lb1 && bear1 && bull0 && o0 <= c1 && c0 >= o1 && (o0 < c1 || c0 > o1),
-         lb1 && bull1 && bear0 && o0 >= c1 && c0 <= o1 && (o0 > c1 || c0 < o1))
-    EMIT(P_cdleveningdojistar, false,                             // :665
-         lb2 && lbull2 && doji1 && fmin(o1, c1) > c2 && bear0 && c0 < (c2 - (b2 * A.pen[PEN_EVENINGDOJISTAR])))
-    EMIT(P_cdleveningstar, false,                                // :703
-         lb2 && lbull2 && short1 && fmin(o1, c1) > c2 && bear0 && c0 < (c2 - (b2 * A.pen[PEN_EVENINGSTAR])))
-    EMIT(P_cdlgapsidesidewhite,                                             // :739
-         lb2 && bull2 && o1 > c2 && bull1 && bull0 && NEAR(b0, b1) && NEAR(o0, o1),
-         lb2 && bear2 && c1 < c2 && bull1 && bull0 && NEAR(b0, b1) && NEAR(o0, o1))
-    EMIT(P_cdlgravestonedoji, false, HAS(f0, CF_DOJI | CF_LUS | CF_VSDS))                         // :777
-    EMIT(P_cdlhammer, lb1 && HAS(f0, CF_SHORT | CF_LDS | CF_VSUS) && bear1, false)                // :802
-    EMIT(P_cdlhangingman, false, lb1 && HAS(f0, CF_SHORT | CF_LDS | CF_VSUS) && bull1)            // :832
-    EMIT(P_cdlharami,                                                      // :862
-         lb1 && lbear1 && bull0 && short0 && o0 > c1 && c0 < o1,
-         lb1 && lbull1 && bear0 && short0 && o0 < c1 && c0 > o1)
-    EMIT(P_cdlharamicross,                                                  // :896
-         lb1 && lbear1 && doji0 && fmax(o0, c0) < o1 && fmin(o0, c0) > c1,
-         lb1 && lbull1 && doji0 && fmax(o0, c0) < c1 && fmin(o0, c0) > o1)
-    EMIT(P_cdlhighwave, HAS(f0, CF_SHORT | CF_LUS | CF_LDS) && bull0, HAS(f0, CF_SHORT | CF_LUS | CF_LDS) && bear0)   // :929
-    {                                                                                              // :956, :987 hikkake / hikkakemod
-        const bool inside12 = h1 < h2 && l1 > l2;
-        EMIT(P_cdlhikkake, lb2 && inside12 && c0 > h2 && bull0, lb2 && inside12 && c0 < l2 && bear0)
-        EMIT(P_cdlhikkakemod,
-             lb3 && (h2 < h3 && l2 > l3) && inside12 && c0 > h3 && bull0, lb3 && (h2 < h3 && l2 > l3) && inside12 && c0 < l3 && bear0)
-    }
-    EMIT(P_cdlhomingpigeon,                                      // :1021
-         lb1 && lbear1 && bear0 && short0 && o0 < o1 && c0 > c1, false)
-    EMIT(P_cdlidentical3crows, false,                           // :1048
-         lb2 && lbear2 && lbear1 && lbear0 && EQUAL(o1, c2) && EQUAL(o0, c1) && (c1 < c2 && c0 < c1))
-    EMIT(P_cdlinneck, false, lb1 && lbear1 && bull0 && o0 < c1 && NEAR(c0, c1))   // :1083
-    EMIT(P_cdlinvertedhammer, lb1 && HAS(f0, CF_SHORT | CF_LUS | CF_VSDS) && bear1, false)        // :1111
-    {                                                                                              // :1141, :1183 kicking / kickingbylength
-        const bool pre = lb1 && maru1 && maru0;
-        const bool bull_kick = pre && bear1 && bull0 && o0 > o1;
-        const bool bear_kick = pre && bull1 && bear0 && o0 < o1;
-        EMIT(P_cdlkicking, bull_kick, bear_kick)
-        EMIT(P_cdlkickingbylength, (bull_kick && b0 >= b1) || (bull_kick && !(bear_kick && b0 >= b1)),
-             (bear_kick && b0 >= b1) || (bear_kick && !(bull_kick && b0 >= b1)))
-    }
-    EMIT(P_cdlladderbottom,    // :1229
-         lb4 && lbear4 && (bear3 && c3 < c4) && (bear2 && c2 < c3) && bear1 && (f1 & CF_LUS) && (bull0 && o0 > o1), false)
-    EMIT(P_cdllongleggeddoji, HAS(f0, CF_DOJI | CF_LUS | CF_LDS), false)                          // :1267
-    EMIT(P_cdllongline, HAS(f0, CF_LONG | CF_SUS | CF_SDS) && bull0, HAS(f0, CF_LONG | CF_SUS | CF_SDS) && bear0)    // :1292
-    EMIT(P_cdlmarubozu, maru0 && bull0, maru0 && bear0)                                           // :1321
-    EMIT(P_cdlmatchinglow, lb1 && lbear1 && bear0 && EQUAL(c0, c1), false) // :1349
-    EMIT(P_cdlmathold,                       // :1376
-         lb4 && lbull4 && (short3 && o3 > c4) && short2 && short1 && (l3 > o4 && l2 > o4 && l1 > o4) && (bull0 && c0 > c4), false)
-    EMIT(P_cdlmorningdojistar,                                    // :1416
-         lb2 && lbear2 && doji1 && fmax(o1, c1) < c2 && bull0 && c0 > (c2 + (b2 * A.pen[PEN_MORNINGDOJISTAR])), false)
-    EMIT(P_cdlmorningstar,                                       // :1454
-         lb2 && lbear2 && short1 && fmax(o1, c1) < c2 && bull0 && c0 > (c2 + (b2 * A.pen[PEN_MORNINGSTAR])), false)
-    EMIT(P_cdlonneck, false, lb1 && lbear1 && bull0 && o0 < c1 && NEAR(c0, l1))   // :1490
-    EMIT(P_cdlpiercing,                                                    // :1519
-         lb1 && lbear1 && bull0 && o0 < c1 && c0 > (c1 + (b1 * A.pen[PEN_PIERCING])) && c0 < o1, false)
-    EMIT(P_cdlrickshawman,                                     // :1553
-         HAS(f0, CF_DOJI | CF_LUS | CF_LDS) && NEAR(us0, ls0), false)
-    EMIT(P_cdlrisefall3methods,               // :1581
-         lb4 && lbull4 && short3 && short2 && short1 && (h3 < h4 && h2 < h4 && h1 < h4 && l3 > l4 && l2 > l4 && l1 > l4) && lbull0 && c0 > c4,
-         lb4 && lbear4 && short3 && short2 && short1 && (h3 < h4 && h2 < h4 && h1 < h4 && l3 > l4 && l2 > l4 && l1 > l4) && lbear0 && c0 < c4)
-    EMIT(P_cdlseparatinglines,                                              // :1647
-         lb1 && lbear1 && lbull0 && EQUAL(o0, o1), lb1 && lbull1 && lbear0 && EQUAL(o0, o1))
-    EMIT(P_cdlshootingstar, false, lb1 && HAS(f0, CF_SHORT | CF_LUS | CF_VSDS) && bull1)          // :1679
-    EMIT(P_cdlshortline, HAS(f0, CF_SHORT | CF_SUS | CF_SDS) && bull0, HAS(f0, CF_SHORT | CF_SUS | CF_SDS) && bear0) // :1709
-    EMIT(P_cdlspinningtop, HAS(f0, CF_SHORT | CF_USGB | CF_LSGB) && bull0, HAS(f0, CF_SHORT | CF_USGB | CF_LSGB) && bear0)  // :1738
-    EMIT(P_cdlstalledpattern, false,                   // :1766
-         lb2 && lbull2 && (lbull1 && c1 > c2) && (bull0 && short0 && c0 > c1) && (o0 > o1 && o0 <= c1))
-    EMIT(P_cdlsticksandwich,                                    // :1797
-         lb2 && lbear2 && lbull1 && o1 > c2 && lbear0 && EQUAL(c0, c2), false)
-    EMIT(P_cdltakuri, HAS(f0, CF_DOJI | CF_VLDS | CF_VSUS), false)                                // :1831
-    EMIT(P_cdltasukigap,          // :1856
-         lb2 && bull2 && bull1 && o1 > c2 && bear0 && o0 > o1 && o0 < c1 && c0 > o2 && c0 < c2,
-         lb2 && bear2 && bear1 && o1 < c2 && bull0 && o0 < o1 && o0 > c1 && c0 < o2 && c0 > c2)
-    EMIT(P_cdlthrusting, false,                                            // :1894
-         lb1 && lbear1 && bull0 && o0 < c1 && c0 > c1 && c0 < (c1 + (b1 * 0.5)))
-    EMIT(P_cdltristar,                                             // :1922
-         lb2 && doji2 && doji1 && doji0 && ((o1 + c1) / 2.0) < ((o2 + c2) / 2.0) && ((o0 + c0) / 2.0) > ((o1 + c1) / 2.0),
-         lb2 && doji2 && doji1 && doji0 && ((o1 + c1) / 2.0) > ((o2 + c2) / 2.0) && ((o0 + c0) / 2.0) < ((o1 + c1) / 2.0))
-    EMIT(P_cdlunique3river,                             // :1964
-         lb2 && lbear2 && (bear1 && l1 < l2 && c1 > l1) && (o1 < o2 && o1 > c2) && (bull0 && short0 && c0 < c1), false)
-    EMIT(P_cdlupsidegap2crows, false,                             // :1997
-         lb2 && lbull2 && (bear1 && o1 > c2 && c1 > c2) && (bear0 && o0 > o1 && c0 > c2 && c0 < c1))
-    EMIT(P_cdlxsidegap3methods,   // :2027
-         lb2 && bull2 && bull1 && o1 > c2 && bear0 && o0 < c1 && o0 > o1 && c0 > o2 && c0 < c2,
-         lb2 && bear2 && bear1 && o1 < c2 && bull0 && o0 > c1 && o0 < o1 && c0 < o2 && c0 > c2)
+#include "candle_patterns.inc"
 #undef EMIT
 #undef HAS
 #undef NEAR
 #undef EQUAL
     (void)pstride; (void)pbase;
+}
+
+// ---- live candle panels (candles_live_host.inc): append bars to a candle panel ------------------------------------
+// A pushed bar's row needs the 4 bars before it and nothing after it, so a live panel keeps the latest CANDLE_HALO bars of
+// each field (the tail) and each thread walks one symbol through the tail and the pushed bars.  Bar-major rows
+// [bar][n_symbols]: a warp's 32 consecutive symbols load one 256-byte line per field and bar and store 128 bytes per
+// Int32 row; price validity is the warp's ballot word, 4 bytes of the bar's LSB-first row bitmap.
+constexpr int CANDLE_LIVE_THREADS = 32;   // one warp per CTA: the few warps of a panel spread evenly over the SMs
+
+struct CandleLiveArgs {
+    const double *rows[4];           // pushed bars of open, high, low, close: [k][n_symbols], or nullptr (unread field: 0.0)
+    const uint32_t *vrows[4];        // their validity words [k][row_words], or nullptr (all valid)
+    const double *tail_in;           // bars T-4 .. T-1: [field][CANDLE_HALO][n_symbols] (0.0 before bar 0)
+    double *tail_out;                // the same after the push, or nullptr (a preview)
+    int32_t *pat[N_PATTERNS];        // Int32 rows [k][n_symbols] or nullptr
+    double *price[N_PRICES];         // f64 rows [k][n_symbols] or nullptr
+    uint32_t *vprice[N_PRICES];      // their validity words [k][row_words]
+    double pen[N_PEN];
+    size_t pat_stride;               // ALL: pattern k's rows = pat[0] + k * pat_stride
+    int n_symbols, k, row_words;
+    int t_base;                      // absolute index of the first pushed bar (the bars before the push, T)
+};
+
+// grid = ceil(n_symbols / CANDLE_LIVE_THREADS).  Every bar is classified once; the pattern block is candle_kernel's text,
+// evaluated at the absolute bar index, so the lookback guards and the zeros before bar 0 are the full panel's.
+template <bool ALL>
+__global__ void __launch_bounds__(CANDLE_LIVE_THREADS) candle_live_kernel(const __grid_constant__ CandleLiveArgs A, const uint64_t pmask) {
+    const int s = blockIdx.x * CANDLE_LIVE_THREADS + threadIdx.x;
+    const bool live = s < A.n_symbols;
+    const size_t n = (size_t)A.n_symbols;
+    const int w = s >> 5;                                    // this warp's validity word in a row
+    auto tail = [&](int f, int j) { return live ? __ldg(A.tail_in + ((size_t)f * CANDLE_HALO + j) * n + s) : 0.0; };
+    double o4 = tail(0, 0), h4 = tail(1, 0), l4 = tail(2, 0), c4 = tail(3, 0);
+    double o3 = tail(0, 1), h3 = tail(1, 1), l3 = tail(2, 1), c3 = tail(3, 1);
+    double o2 = tail(0, 2), h2 = tail(1, 2), l2 = tail(2, 2), c2 = tail(3, 2);
+    double o1 = tail(0, 3), h1 = tail(1, 3), l1 = tail(2, 3), c1 = tail(3, 3);
+    unsigned f4 = classify(o4, h4, l4, c4), f3 = classify(o3, h3, l3, c3), f2 = classify(o2, h2, l2, c2),
+             f1 = classify(o1, h1, l1, c1);
+    const double nn = __longlong_as_double(0x7ff8000000000000LL);
+    for (int t = 0; t < A.k; ++t) {
+        const int i = A.t_base + t;                          // absolute bar index
+        const size_t at = (size_t)t * n + s;
+        double o0 = 0.0, h0 = 0.0, l0 = 0.0, c0 = 0.0;
+        if (live) {
+            if (A.rows[0]) o0 = __ldg(A.rows[0] + at);
+            if (A.rows[1]) h0 = __ldg(A.rows[1] + at);
+            if (A.rows[2]) l0 = __ldg(A.rows[2] + at);
+            if (A.rows[3]) c0 = __ldg(A.rows[3] + at);
+        }
+        const unsigned f0 = classify(o0, h0, l0, c0);
+        {
+            unsigned vo = 0xffffffffu, vh = vo, vl = vo, vc = vo;
+            const size_t wi = (size_t)t * A.row_words + w;
+            if (live) {
+                if (A.vrows[0]) vo = __ldg(A.vrows[0] + wi);
+                if (A.vrows[1]) vh = __ldg(A.vrows[1] + wi);
+                if (A.vrows[2]) vl = __ldg(A.vrows[2] + wi);
+                if (A.vrows[3]) vc = __ldg(A.vrows[3] + wi);
+            }
+            const unsigned bit = 1u << (threadIdx.x & 31);
+            const bool ko = vo & bit, kh = vh & bit, kl = vl & bit, kc = vc & bit;
+            auto emit = [&](int k, double v, bool ok) {
+                if (!A.price[k]) return;
+                ok = ok && live;
+                const unsigned m = __ballot_sync(0xffffffffu, ok);
+                if (live) {
+                    A.price[k][at] = ok ? v : nn;
+                    if ((threadIdx.x & 31) == 0 && A.vprice[k]) A.vprice[k][wi] = m;
+                }
+            };
+#include "candle_prices.inc"
+        }
+        if (ALL || pmask) {
+            int32_t *const pbase = A.pat[0] + at;
+            const size_t pstride = A.pat_stride;
+#define HAS(f, m) (((f) & (m)) == (m))
+#define NEAR(a, b) (fabs((a) - (b)) < near_t)
+#define EQUAL(a, b) (fabs((a) - (b)) < equal_t)
+#define EMIT(id, up, dn)                                                                                  \
+    if (ALL || (pmask >> (id) & 1)) {                                                                     \
+        if (live) *(ALL ? pbase + (size_t)(id) * pstride : A.pat[id] + at) = (up) ? 100 : ((dn) ? -100 : 0); \
+    }
+#include "candle_patterns.inc"
+#undef EMIT
+#undef HAS
+#undef NEAR
+#undef EQUAL
+            (void)pstride; (void)pbase;
+        }
+        o4 = o3; h4 = h3; l4 = l3; c4 = c3; f4 = f3;
+        o3 = o2; h3 = h2; l3 = l2; c3 = c2; f3 = f2;
+        o2 = o1; h2 = h1; l2 = l1; c2 = c1; f2 = f1;
+        o1 = o0; h1 = h0; l1 = l0; c1 = c0; f1 = f0;
+    }
+    if (A.tail_out && live) {
+        auto put = [&](int j, double o, double h, double l, double c) {
+            A.tail_out[((size_t)0 * CANDLE_HALO + j) * n + s] = o;
+            A.tail_out[((size_t)1 * CANDLE_HALO + j) * n + s] = h;
+            A.tail_out[((size_t)2 * CANDLE_HALO + j) * n + s] = l;
+            A.tail_out[((size_t)3 * CANDLE_HALO + j) * n + s] = c;
+        };
+        put(0, o4, h4, l4, c4);
+        put(1, o3, h3, l3, c3);
+        put(2, o2, h2, l2, c2);
+        put(3, o1, h1, l1, c1);
+    }
 }
 
 // synthetic candle panel for the bench (device-side, counter-based): a random walk of opens with bodies and

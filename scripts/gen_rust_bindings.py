@@ -19,7 +19,7 @@ BEGIN, END = "<!-- BEGIN GENERATED: rust bindings of include/pqb200.h -->", "<!-
 
 SCALARS = {"int": "c_int", "int32_t": "i32", "int64_t": "i64", "uint32_t": "u32", "uint64_t": "u64", "double": "f64",
            "float": "f32", "uint8_t": "u8", "int8_t": "i8", "char": "c_char", "void": "c_void", "size_t": "usize"}
-OPAQUE = ["pqb_engine", "pqb_panel", "pqb_multi", "pqb_candles", "pqb_split", "pqb_long", "pqb_windows", "pqb_live", "ArrowArray", "ArrowSchema"]
+OPAQUE = ["pqb_engine", "pqb_panel", "pqb_multi", "pqb_candles", "pqb_split", "pqb_long", "pqb_windows", "pqb_live", "pqb_windows_live", "pqb_candles_live", "ArrowArray", "ArrowSchema"]
 
 
 def camel(name: str) -> str:

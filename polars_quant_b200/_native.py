@@ -60,6 +60,12 @@ class CandleParams(C.Structure):
                 ("pen_morningdojistar", C.c_double), ("pen_morningstar", C.c_double), ("pen_piercing", C.c_double)]
 
 
+class LiveScreen(C.Structure):
+    """pqb_live_screen: what a live panel's screen serves (include/pqb200.h "live screens")."""
+    _fields_ = [("oversold", C.c_double), ("overbought", C.c_double), ("ma_type", C.c_int32), ("ma_fast", C.c_int32),
+                ("ma_slow", C.c_int32), ("info", C.c_int32)]
+
+
 N_PATTERNS = 61
 N_PRICES = 5
 PRICE_NAMES = ["avgprice", "medprice", "typprice", "wclprice", "bop"]
@@ -289,6 +295,17 @@ def lib() -> C.CDLL:
                                          C.POINTER(C.c_void_p)]
         L.pqb_live_host_voided.argtypes = [C.c_void_p, C.c_int]
         L.pqb_live_host_voided.restype = C.c_void_p
+        L.pqb_live_screen_default.argtypes = [C.POINTER(LiveScreen)]
+        L.pqb_live_screen_default.restype = None
+        L.pqb_live_create_screen.argtypes = [C.c_void_p, C.POINTER(SuiteParams), C.c_uint64, C.c_int64, C.c_uint32,
+                                             C.POINTER(LiveScreen), C.POINTER(C.c_void_p)]
+        L.pqb_live_host_signal.argtypes = [C.c_void_p, C.c_int]
+        L.pqb_live_host_signal.restype = C.c_void_p
+        L.pqb_live_host_info.argtypes = [C.c_void_p]
+        L.pqb_live_host_info.restype = C.c_void_p
+        L.pqb_live_host_info_valid.argtypes = [C.c_void_p]
+        L.pqb_live_host_info_valid.restype = C.c_void_p
+        L.pqb_live_info.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 

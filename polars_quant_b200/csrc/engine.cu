@@ -2503,5 +2503,6 @@ extern "C" int pqb_multi_run_host(pqb_multi *m, const pqb_suite_params *params) 
 #include "signals_host.inc"
 #include "info_host.inc"
 #include "live_host.inc"
+#include "live_screen_host.inc"
 #include "windows_live_host.inc"
 #include "candles_live_host.inc"

@@ -459,12 +459,14 @@ class WidePanel:
 
     # ---- live: append new rows to the computed table ----
     def live(self, params: N.SuiteParams | None = None, outputs=None, max_push_bars: int = 64, devices=None,
-             nulls: bool = False) -> "WideLive":
+             nulls: bool = False, screen=None) -> "WideLive":
         """A live panel primed from this table (include/pqb200.h "live panels"): `.push(rows)` takes k new rows in the
         table's own `date` + `{symbol}_{field}` shape and returns `date` + `{symbol}_{output}` for those rows -- the
         columns, names and values `suite()` of the concatenated table gives for them.  One GPU (`devices` is refused).
         nulls=True: the table and the pushed rows may have halted cells; after each push `WideLive.voided` lists the
-        `{symbol}_{output}` columns whose earlier rows that push turned null."""
+        `{symbol}_{output}` columns whose earlier rows that push turned null.  screen (see LivePanel): after each push
+        `WideLive.signals` holds `date` + `{symbol}_{signal}` Int8 columns, and `WideLive.info()` equals `info()` of the
+        concatenated table."""
         if devices:
             raise NotImplementedError("live panels run on one GPU: multi-GPU live panels are not built")
         symbols, cols = split_columns(self.table, SUITE_FIELDS)
@@ -481,10 +483,18 @@ class WidePanel:
             N.check(N.lib().pqb_panel_set_record_batch(p._h, C.byref(arr), C.byref(sch), sym.ctypes.data, fld.ctypes.data, 0))
             p.upload()
             from .live import LivePanel
-            lp = LivePanel(p, params, omask, max_push_bars, nulls=nulls)
+            lp = LivePanel(p, params, omask, max_push_bars, nulls=nulls, screen=screen)
         finally:
             p.close()
-        return WideLive(lp, symbols, {f: cols[f] for f in SUITE_FIELDS}, sorted(names, key=N.OUTPUT_NAMES.index))
+        wl = WideLive(lp, symbols, {f: cols[f] for f in SUITE_FIELDS}, sorted(names, key=N.OUTPUT_NAMES.index))
+        if lp.screen is not None and lp.screen.info:
+            # info() lists symbols in the order of the table's close / high / low / volume / open columns
+            info_syms, ocols = split_columns(self.table, SUITE_FIELDS + ("open",))
+            wl._info_order = [symbols.index(s) for s in info_syms if s in wl._index]
+            wl._open_cols = ocols["open"]
+            last = self.n_bars - 1
+            wl._open = [self._col(ocols["open"][s])[last].as_py() if s in ocols["open"] else None for s in symbols]
+        return wl
 
     # ---- Selector.info(): last-row reductions (README.md:832-851) ----
     def info(self) -> pa.Table:
@@ -568,6 +578,9 @@ class WideLive:
     def __init__(self, live, symbols, cols, outputs):
         self.live, self.symbols, self._cols, self.outputs = live, symbols, cols, outputs
         self.voided: list[str] = []             # `{symbol}_{output}` columns whose earlier rows the last push made null
+        self.signals: pa.Table | None = None    # screen: `date` + `{symbol}_{signal}` of the last push
+        self._index = {s: j for j, s in enumerate(symbols)}
+        self._info_order, self._open_cols, self._open = None, {}, []
 
     @property
     def bars(self) -> int:
@@ -596,4 +609,33 @@ class WideLive:
         out = pa.table(out_cols, names=out_names)
         if "date" in index:
             out = out.add_column(0, "date", rows.column(index["date"]))
+        if self.live.screen is not None:
+            sig_cols, sig_names = [], []
+            for j, s in enumerate(self.symbols):
+                for name, a in self.live.signals.items():
+                    sig_cols.append(pa.array(a[j], type=pa.int8()))
+                    sig_names.append("%s_%s" % (s, name))
+            self.signals = pa.table(sig_cols, names=sig_names)
+            if "date" in index:
+                self.signals = self.signals.add_column(0, "date", rows.column(index["date"]))
+            if commit and self._info_order is not None:
+                self._open = [rows.column(index[self._open_cols[s]])[k - 1].as_py() if self._open_cols.get(s) in index else None
+                              for s in self.symbols]
         return out
+
+    def info(self) -> pa.Table:
+        """`WidePanel.info()` of the table with every committed push appended: one row per symbol, the README's 15
+        `Selector.info()` columns (`open` from the last committed row's `{symbol}_open`, null when it has none).  Needs a
+        screen with info."""
+        if self._info_order is None:
+            raise ValueError("info() needs a live table created with screen info (screen=True or dict(info=True))")
+        res = self.live.info()
+        order = self._info_order
+        out = {"symbol": pa.array([self.symbols[j] for j in order]),
+               "open": pa.array([self._open[j] for j in order], type=pa.float64())}
+        for name in N.INFO_NAMES:
+            v, ok = res[name]
+            out[name] = pa.array(v[order], mask=~ok[order])
+        names = ["symbol", "price", "open", "high", "low", "volume", "return_1d", "return_5d", "return_20d", "volatility",
+                 "ma_5", "ma_10", "ma_20", "volume_ratio", "amplitude"]
+        return pa.table([out[n] for n in names], names=names)
